@@ -11,11 +11,17 @@ kernel, GCN degree scalings fused; layer 1 reads one shared X, layers 2-3 read p
 [S,N,D] activations) and one fused backward launch (transposed aggregation dX over the
 regenerated noise).  edge-samples per step = E * S * 3.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--mode mle|vi]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--mode mle|vi] [--dump-outputs DIR]
 
 N > 1: launched by torchrun, one rank per GPU; the MC samples are the sharded unit (rank r
 draws Philox sample indices [r*S, (r+1)*S)), no data-path collective, weak scaling.
 Prints ONE JSON line on rank 0.
+
+--dump-outputs DIR writes what the last timed step computed as DIR/<name>.npy (float32), on
+rank 0: the outputs of the three layers (out1..out3) and the input gradient dx, each [S, R, D]
+over a fixed node sample R (see dump_rows), plus dparams [3, 2] (d loc, d scale per layer) in vi
+mode; for --impl reference, out and dx [R, D] of its one layer pass.  The inputs depend only on
+the arguments, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import ctypes
@@ -54,6 +60,20 @@ def synth_graph(seed=0x57A6 + 2):
         ids = rng.choice(N_NODES, size=N_EDGES, p=p)
         return rng.permutation(N_NODES)[ids]
     return endpoints().astype(np.int64), endpoints().astype(np.int64)
+
+
+def dump_rows(src, dst, n_random=1024, n_hubs=32):
+    """Node rows kept by --dump-outputs (the full [S, N, D] outputs are 1.39 GB each): a seeded uniform
+    sample plus the highest in- and out-degree nodes, whose rows take the hub code paths of the kernels."""
+    rng = np.random.default_rng(0xD0)
+    hubs = [np.argsort(np.bincount(e, minlength=N_NODES), kind="stable")[-n_hubs:] for e in (dst, src)]
+    return np.unique(np.concatenate([rng.choice(N_NODES, n_random, replace=False)] + hubs))
+
+
+def dump_outputs(out_dir, arrays):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
 
 
 def peaks():
@@ -138,6 +158,9 @@ def run_reference(args, rank):
     for k in range(args.steps):
         lp.run(args.warmup + k)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        rows = dump_rows(src, dst)
+        dump_outputs(args.dump_outputs, {"out": lp.out[rows], "dx": lp.dx[rows]})
     val = N_EDGES * args.steps / dt / 1e9
     sample = "1 layer x 1 MC sample fwd+bwd per step at the full arxiv shape (noise tensor materialised, as the reference does)"
     line = {"impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus,
@@ -383,6 +406,13 @@ def run_ours(args, rank, world):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
     launches = int(path.lib.stag_launch_count() - launches0)   # counted inside libstag_b200.so
+    if args.dump_outputs and rank == 0:
+        rows = torch.from_numpy(dump_rows(src, dst)).to(dev)
+        arrays = {"out%d" % (i + 1): a.index_select(1, rows).cpu().numpy() for i, a in enumerate(path.act)}
+        arrays["dx"] = path.dx0.index_select(1, rows).cpu().numpy()
+        if vi:
+            arrays["dparams"] = path.dp.reshape(N_LAYERS, 2).cpu().numpy()
+        dump_outputs(args.dump_outputs, arrays)
     ms_per_step = ms / args.steps
     edge_samples = N_EDGES * S * N_LAYERS * world
     value = edge_samples / (ms_per_step * 1e-3) / 1e9
@@ -477,7 +507,11 @@ def main():
     ap.add_argument("--normal", default="hadamard", choices=["hadamard", "boxmuller"],
                     help="standard-normal generator of the fused kernels: tensor-core Walsh-Hadamard mix "
                          "(agg_wh_quad_kernel) or 16-bit Box-Muller (agg_stream_kernel)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (float32, a fixed node sample)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     if args.impl == "reference":
