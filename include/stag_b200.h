@@ -203,6 +203,41 @@ STAG_API int stag_spmm_bwd(const StagGraph* csr, const float* x, int64_t ldx, in
                   float* dparam0, float* dparam1, float* dw_external,
                   void* ws, size_t ws_bytes, void* stream);
 
+/* ---- fused stochastic MAX aggregation ---------------------------------------------------
+ * Forward (CSC graph), replaces rsample_noise + relu + update_all(u_mul_e, fn.max) (GraphSAGE 'pool', GIN 'max'):
+ *
+ *   out[s,v,c] = max_{j in row v} w_s[eid_j, c] * x[s,u_j,c]        (fp32 product, then compare)
+ *   arg[s,v,c] = eid_j of the winning edge (ORIGINAL edge id)
+ *
+ * Ties go to the first edge in stored order, i.e. the smallest edge id (strict >, the CSC is a stable sort); rows
+ * without in-edges get out = 0, arg = -1.  arg has the strides of out.  The noise is the stream stag_noise_emit writes
+ * for the same spec (every kind; K == 1 or D, STAG_NOISE_NORMAL_HADAMARD with K == D), so the result equals the max over
+ * the materialised tensor bit for bit.  No degree scalings; in_norm and STAG_PARAM_EDGE_CHANNEL are rejected
+ * (STAG_EINVAL): materialise the noise for those.  Same workspace as stag_spmm_fwd (stag_spmm_workspace_bytes).
+ */
+STAG_API int stag_spmm_max_fwd(const StagGraph* g, const float* x, int64_t ldx, int64_t x_sample_stride,
+                      int32_t D, int32_t S, const StagNoise* noise,
+                      float* out, int32_t* arg, int64_t ldo, int64_t out_sample_stride,
+                      void* ws, size_t ws_bytes, void* stream);
+
+/* Backward of stag_spmm_max_fwd (CSR graph; arg = the forward's, at the strides of dout).  Only the winner of a
+ * (sample, row, channel) receives its gradient:
+ *   dx[s,u,c]  = sum_j [arg[s,v_j,c] == eid_j] w_s[eid_j,c] * dout[s,v_j,c]
+ *   dw[s,e,c]  = [arg[s,v,c] == e] x[s,u,c] * dout[s,v,c]      (never stored unless EXTERNAL and dw_external != NULL:
+ *                                                             K == D per channel, K == 1 summed over the channels)
+ *   NORMAL : dparam0 = sum dw (d loc), dparam1 = sum dw*eps (d scale)
+ *   UNIFORM: dparam0 = sum dw*(1-u) (d low), dparam1 = sum dw*u (d high)        (relu: masked by w > 0)
+ * dx, dparam0/1 and dw_external are each optional (NULL).  SCALAR / CHANNEL parameter gradients OVERWRITE dparam*,
+ * EDGE ([E,1]) ones ACCUMULATE (summed over the S samples); per-edge outputs need a graph built with erow.
+ * Deterministic: no float atomics.
+ */
+STAG_API int stag_spmm_max_bwd(const StagGraph* csr, const float* x, int64_t ldx, int64_t x_sample_stride,
+                      const float* dout, const int32_t* arg, int64_t ldg, int64_t dout_sample_stride,
+                      int32_t D, int32_t S, const StagNoise* noise,
+                      float* dx, int64_t lddx, int64_t dx_sample_stride,
+                      float* dparam0, float* dparam1, float* dw_external,
+                      void* ws, size_t ws_bytes, void* stream);
+
 /* Materialise the noise tensor w [S,E,K] (original edge order) from the same Philox stream
  * the fused kernels use: compatibility path for base layers that are not fused
  * (StagLayer._edge_weight_sample, stag/layers.py:107; KL fallback :141-143) and for RNG tests.

@@ -79,6 +79,9 @@ SIGNATURES = {
     "stag_spmm_fwd": (_I, [_GP, _V, _I64, _I64, _I32, _I32, _NP, _V, _V, _V, _I64, _I64, _V, _V, _SZ, _V]),
     "stag_spmm_bwd": (_I, [_GP, _V, _I64, _I64, _V, _I64, _I64, _I32, _I32, _NP, _V, _V, _V, _I64, _I64,
                            _V, _V, _V, _V, _SZ, _V]),
+    "stag_spmm_max_fwd": (_I, [_GP, _V, _I64, _I64, _I32, _I32, _NP, _V, _V, _I64, _I64, _V, _SZ, _V]),
+    "stag_spmm_max_bwd": (_I, [_GP, _V, _I64, _I64, _V, _V, _I64, _I64, _I32, _I32, _NP, _V, _I64, _I64,
+                               _V, _V, _V, _V, _SZ, _V]),
     "stag_noise_emit": (_I, [_NP, _I64, _I32, _V, _V, _V]),
     "stag_noise_kl_workspace_bytes": (_SZ, [_I32]),
     "stag_noise_kl": (_I, [_NP, _I64, _I32, ctypes.POINTER(StagPrior), _V, _V, _V, _V, _SZ, _V]),

@@ -2424,3 +2424,4 @@ extern "C" int stag_segment_reduce(const float* feat, int64_t ldf, const int32_t
   STAG_LAUNCH_CHECK();
   return STAG_OK;
 }
+#include "spmm_max.cuh"

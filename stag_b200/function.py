@@ -2,7 +2,8 @@
 
 Covers the builtins the reference uses: ``fn.u_mul_e`` / ``fn.copy_src`` (copy_u) /
 ``fn.copy_edge`` (copy_e) with ``fn.sum`` / ``fn.mean`` (stag/layers.py:12-15;
-stag/zoo/gcn.py:59,63,95; stag/zoo/graph_sage.py:53,57,72,86; stag/zoo/gated_gcn.py:30-42)
+stag/zoo/gcn.py:59,63,95; stag/zoo/graph_sage.py:53,57,72,86; stag/zoo/gated_gcn.py:30-42),
+``fn.max`` / ``fn.min`` (SAGEConv 'pool', GINConv 'max'; ties go to the first edge in edge-id order)
 and ``fn.u_add_v`` for ``apply_edges`` (stag/zoo/gat.py:114).
 """
 import torch
@@ -63,10 +64,18 @@ def mean(msg, out):
     return Reduce("mean", msg, out)
 
 
+def max(msg, out):  # noqa: A001
+    return Reduce("max", msg, out)
+
+
+def min(msg, out):  # noqa: A001
+    return Reduce("min", msg, out)
+
+
 def run(g, message, reduce):
     """update_all(message, reduce) on the CUDA kernels."""
     from . import ops
-    if reduce.kind not in ("sum", "mean"):
+    if reduce.kind not in ("sum", "mean", "max", "min"):
         raise NotImplementedError("reduce %r" % reduce.kind)
     if message.kind == "copy_u":
         x = g.ndata[message.a]

@@ -396,8 +396,14 @@ def stochastic_aggregate(graph, feat, edge_weight=None, reduce="sum", src_scale=
 
     feat ``[N,D]`` -> out ``[N,D]`` (or ``[S,N,D]`` when ``n_samples=S`` shares feat over S
     Monte-Carlo samples); feat ``[S,N,D]`` -> out ``[S,N,D]``.  ``reduce='mean'`` divides
-    by clamp(in_degree, 1) (dgl fn.mean).
+    by clamp(in_degree, 1) (dgl fn.mean).  ``reduce='max'`` / ``'min'`` take the max / min of the
+    messages w * feat[u] instead (dgl fn.max / fn.min): ties go to the first edge in edge-id order,
+    which alone receives the gradient; rows without in-edges are 0.  No scales with max / min.
     """
+    if reduce not in ("sum", "mean", "max", "min"):
+        raise ValueError("reduce must be 'sum', 'mean', 'max' or 'min'; got %r" % (reduce,))
+    if reduce in ("max", "min") and (src_scale is not None or dst_scale is not None):
+        raise ValueError("reduce=%r takes no src_scale / dst_scale" % (reduce,))
     g = as_graph(graph)
     st = g._s
     N, E = st.num_nodes, st.num_edges
@@ -414,11 +420,15 @@ def stochastic_aggregate(graph, feat, edge_weight=None, reduce="sum", src_scale=
     if feat.shape[-2] != st.num_src:
         raise ValueError("feat has %d rows, graph has %d source nodes" % (feat.shape[-2], st.num_src))
     D = feat.shape[-1]
+    if reduce in ("max", "min"):
+        if reduce == "min":  # min_e w x = -max_e w (-x): ties go to the first minimum
+            out = -_aggregate_max(g, -feat, edge_weight, S, shared)
+        else:
+            out = _aggregate_max(g, feat, edge_weight, S, shared)
+        return out[0] if squeeze else out
     if reduce == "mean":
         m = st.scale(True, "inv")
         dst_scale = m if dst_scale is None else dst_scale * m
-    elif reduce != "sum":
-        raise ValueError("reduce must be 'sum' or 'mean'")
     cfg = {"graph": g, "S": S, "shared": shared, "relu": False, "in_norm": False, "sample_base": 0,
            "seed": 0, "offset": 0, "param_shape": _lib.PARAM_SCALAR, "K": D,
            "src_scale": _c(src_scale), "dst_scale": _c(dst_scale)}
@@ -476,6 +486,139 @@ def stochastic_aggregate(graph, feat, edge_weight=None, reduce="sum", src_scale=
         ext = w
     out = _StochasticSpMM.apply(feat, p0, p1, ext, cfg)
     return out[0] if squeeze else out
+
+
+class _StochasticMax(torch.autograd.Function):
+    """stag_spmm_max_fwd / stag_spmm_max_bwd: out[s,v,c] = max over the in-edges of w * feat[u], with the winning edge
+    id kept for the backward (only the winner receives the gradient)."""
+
+    @staticmethod
+    def forward(ctx, feat, p0, p1, ext, cfg):
+        g = cfg["graph"]
+        st = g._s
+        dev = feat.device
+        lib = _lib.load()
+        S, shared = cfg["S"], cfg["shared"]
+        N, NS, D = st.num_nodes, st.num_src, feat.shape[-1]
+        x = _c(feat)
+        p0c, p1c, extc = _c(p0), _c(p1), _c(ext)
+        out = torch.empty((S, N, D), dtype=torch.float32, device=dev)
+        arg = torch.empty((S, N, D), dtype=torch.int32, device=dev)
+        with _on_device(dev):
+            csc, _ = st.csx(True)
+            ws = _workspace(st, lib, csc, True, D, S)
+            nz = _fill_noise(None, cfg["kind"], cfg["K"], p0c, p1c, extc, cfg["relu"], False, cfg["sample_base"],
+                             cfg["seed"], cfg["offset"], cfg["param_shape"])
+            _lib.check(lib.stag_spmm_max_fwd(
+                ctypes.byref(csc), x.data_ptr(), D, 0 if shared else NS * D, D, S, ctypes.byref(nz),
+                out.data_ptr(), arg.data_ptr(), D, N * D, ws.data_ptr(), ws.numel(), _stream(dev)))
+        ctx.cfg = cfg
+        ctx.feat_shape = feat.shape
+        ctx.param_shapes = (None if p0 is None else p0.shape, None if p1 is None else p1.shape)
+        ctx.ext_shape = None if ext is None else ext.shape
+        need_x = any(ctx.needs_input_grad[1:4])
+        ctx.save_for_backward(x if need_x else None, p0c, p1c, extc, arg)
+        return out
+
+    @staticmethod
+    def backward(ctx, gout):
+        cfg = ctx.cfg
+        st = cfg["graph"]._s
+        x, p0c, p1c, extc, arg = ctx.saved_tensors
+        lib = _lib.load()
+        dev = gout.device
+        S, shared = cfg["S"], cfg["shared"]
+        N, NS, D, K = st.num_nodes, st.num_src, gout.shape[-1], cfg["K"]
+        need_dx = ctx.needs_input_grad[0]
+        need_dp = (ctx.needs_input_grad[1] or ctx.needs_input_grad[2]) and cfg["kind"] in (
+            _lib.NOISE_NORMAL, _lib.NOISE_UNIFORM)
+        need_dext = ctx.needs_input_grad[3] and cfg["kind"] == _lib.NOISE_EXTERNAL
+        gout = gout.to(torch.float32).contiguous()
+        dx = torch.empty((S, NS, D), dtype=torch.float32, device=dev) if need_dx else None
+        dext = torch.empty((S, st.num_edges, K), dtype=torch.float32, device=dev) if need_dext else None
+        dp0 = dp1 = None
+        if need_dp:
+            n = {_lib.PARAM_SCALAR: 1, _lib.PARAM_CHANNEL: K, _lib.PARAM_EDGE: st.num_edges}[cfg["param_shape"]]
+            dp0 = torch.zeros(n, dtype=torch.float32, device=dev)
+            dp1 = torch.zeros(n, dtype=torch.float32, device=dev)
+        if need_dx or need_dp or need_dext:
+            with _on_device(dev):
+                csr, _ = st.csx(False)
+                ws = _workspace(st, lib, csr, False, D, S)
+                nz = _fill_noise(None, cfg["kind"], K, p0c, p1c, extc, cfg["relu"], False, cfg["sample_base"],
+                                 cfg["seed"], cfg["offset"], cfg["param_shape"])
+                _lib.check(lib.stag_spmm_max_bwd(
+                    ctypes.byref(csr), _ptr(x), D, 0 if shared else NS * D, gout.data_ptr(), arg.data_ptr(), D, N * D,
+                    D, S, ctypes.byref(nz), _ptr(dx), D, NS * D, _ptr(dp0), _ptr(dp1), _ptr(dext),
+                    ws.data_ptr(), ws.numel(), _stream(dev)))
+        gfeat = gp0 = gp1 = gext = None
+        if need_dx:
+            gfeat = (dx.sum(0) if shared else dx).reshape(ctx.feat_shape)
+        if need_dp:
+            s0, s1 = ctx.param_shapes
+            if ctx.needs_input_grad[1]:
+                gp0 = dp0.reshape(s0) if dp0.numel() == max(1, _numel(s0)) else dp0.reshape(-1).sum_to_size(s0)
+            if ctx.needs_input_grad[2] and s1 is not None:
+                gp1 = dp1.reshape(s1) if dp1.numel() == max(1, _numel(s1)) else dp1.reshape(-1).sum_to_size(s1)
+        if need_dext:
+            gext = dext.reshape(ctx.ext_shape) if dext.numel() == _numel(ctx.ext_shape) else dext
+        return gfeat, gp0, gp1, gext, None
+
+
+def _aggregate_max(g, feat, edge_weight, S, shared):
+    """[S,N,D] max over the in-edges of w * feat[u] (see :func:`stochastic_aggregate`).  In-norm specs and [E,K]
+    parameters go through the materialised noise tensor (differentiable through _NoiseEmit): the in-norm scale of
+    Normal noise can be negative and flip the max, and the fused kernels take neither."""
+    st = g._s
+    E, D = st.num_edges, feat.shape[-1]
+    cfg = {"graph": g, "S": S, "shared": shared, "relu": False, "sample_base": 0, "seed": 0, "offset": 0,
+           "param_shape": _lib.PARAM_SCALAR, "K": D, "kind": _lib.NOISE_NONE}
+    if isinstance(edge_weight, NoiseSpec):
+        spec = edge_weight
+        if spec.num_edges != E:
+            raise ValueError("noise spec was made for %d edges, graph has %d" % (spec.num_edges, E))
+        if spec.K not in (1, D):
+            raise ValueError("noise width K=%d must be 1 or feat width %d" % (spec.K, D))
+        if spec.in_norm or spec.param_shape == _lib.PARAM_EDGE_CHANNEL:
+            w = spec.materialize(n_samples=S)                                   # [S,E,K], relu applied
+            if spec.in_norm:
+                from .layers import _in_norm
+                w = torch.stack([_in_norm(g, w[s]) for s in range(S)])
+            return _aggregate_max(g, feat, w, S, shared)
+        cfg.update(kind=spec.lib_kind, K=spec.K, relu=spec.relu, sample_base=spec.sample_base, seed=spec.seed,
+                   offset=spec.offset, param_shape=spec.param_shape)
+        p0, p1 = spec.p0, spec.p1
+        Dp = D
+        if cfg["kind"] == _lib.NOISE_NORMAL_HADAMARD and D % 128:
+            Dp = spec.hadamard_width                        # the tensor-core stream comes in groups of 128 channels
+        elif D % 4 and D > 128 and spec.K == D:
+            Dp = D + (-D) % 4                               # 16-byte rows for the vector loads (as the sum path)
+        if Dp != D:
+            if spec.K == D:
+                cfg["K"] = Dp
+                if spec.param_shape == _lib.PARAM_CHANNEL:
+                    p0 = torch.nn.functional.pad(p0, (0, Dp - D))
+                    p1 = None if p1 is None else torch.nn.functional.pad(p1, (0, Dp - D), value=1.0)
+            featp = torch.nn.functional.pad(feat, (0, Dp - D))
+            return _StochasticMax.apply(featp, p0, p1, None, cfg)[..., :D]
+        return _StochasticMax.apply(feat, p0, p1, None, cfg)
+    if edge_weight is None:
+        return _StochasticMax.apply(feat, None, None, None, cfg)
+    w = edge_weight
+    _require_cuda(w, "edge_weight")
+    if w.dim() == 1:
+        w = w.unsqueeze(-1)
+    K = w.shape[-1]
+    if K not in (1, D):
+        raise ValueError("edge_weight width %d must be 1 or feat width %d" % (K, D))
+    if w.dim() == 2:
+        if w.shape[0] != E:
+            raise AssertionError("edge_weight has %d rows, graph has %d edges" % (w.shape[0], E))
+        w = w.unsqueeze(0).expand(S, E, K)
+    elif w.dim() != 3 or w.shape[0] != S or w.shape[1] != E:
+        raise ValueError("edge_weight must be [E,K] or [S,E,K]; got %s" % (tuple(edge_weight.shape),))
+    cfg.update(kind=_lib.NOISE_EXTERNAL, K=K)
+    return _StochasticMax.apply(feat, None, None, w, cfg)
 
 
 class _HeadsAggregate(torch.autograd.Function):

@@ -1,5 +1,5 @@
 """``GIN`` -- the reference's ``stag.zoo.GIN`` (stag/zoo/gin.py:1-11): ``dgl.nn.GINConv``
-with a Linear ``apply_func``; ``rst = apply_func((1 + eps) * h_v + sum_e w * h_u)``."""
+with a Linear ``apply_func``; ``rst = apply_func((1 + eps) * h_v + agg_e w * h_u)``, agg = sum, mean or max."""
 import torch
 from torch import nn
 
@@ -14,7 +14,7 @@ class GIN(nn.Module):
     def __init__(self, in_features, out_features, aggregator_type="sum", init_eps=0, learn_eps=False,
                  activation=None):
         super().__init__()
-        if aggregator_type not in ("sum", "mean"):
+        if aggregator_type not in ("sum", "mean", "max"):
             raise NotImplementedError("stag_b200.zoo.GIN: aggregator_type=%r" % aggregator_type)
         self.apply_func = nn.Linear(in_features, out_features)
         self._aggregator_type = aggregator_type
