@@ -291,6 +291,31 @@ STAG_API int stag_attention_softmax_bwd(const StagGraph* csc, const float* el, c
                                int32_t H, const float* a, const float* da, float* dw, float* dpre, float* d_er,
                                void* stream);
 
+/* The same over S Monte-Carlo samples in one launch, with the logit noise drawn inside the kernel (stochastic GAT):
+ *   logit[s,e,h] = w_s[e,h] * leaky_relu(el[s,u_e,h] + er[s,v_e,h], slope),   a[s,e,h] = softmax over the in-edges of v_e
+ * el / er: sample s at el + s * el_sample_stride (0: one [num_cols,H] / [num_rows,H] shared by every sample, the first
+ * layer); a [S,E,H] in original edge order.  noise: STAG_NOISE_NONE, EXTERNAL ([S,E,H]) or a generated kind (NORMAL,
+ * UNIFORM, BERNOULLI) with K == H, any parameter shape, relu, sample_base and the device counter.  The variate of
+ * (edge, head h, sample s) is the one stag_noise_emit writes for channel h of sample sample_base + s, so the result
+ * equals the attention over the materialised tensor bit for bit.  STAG_NOISE_NORMAL_HADAMARD -> STAG_EUNSUPPORTED,
+ * in_norm -> STAG_EINVAL (materialise the noise for those).
+ * Backward from da [S,E,H]: dpre [S,E,H] = d(el[u] + er[v]) per edge (the caller sums it per SOURCE on the CSR graph),
+ * d_er [S,num_rows,H] = its sum per destination, dw_external [S,E,H] (EXTERNAL only, may be NULL) and, for Normal /
+ * Uniform noise, dparam0 / dparam1 (both or neither) in the parameter shape: d loc / d scale, d low / d high, masked by
+ * w > 0 under relu.  SCALAR / CHANNEL results OVERWRITE dparam* and are summed over the S samples; EDGE ([E,1], summed
+ * over the heads) and EDGE_CHANNEL ([E,H]) results ACCUMULATE (the caller zeroes them once).  The workspace holds the
+ * per-CTA partials of the SCALAR / CHANNEL reduction (stag_attention_workspace_bytes; unused otherwise).  No float
+ * atomics: bitwise run-to-run. */
+STAG_API size_t stag_attention_workspace_bytes(const StagGraph* csc, int32_t H, int32_t S);
+STAG_API int stag_attention_softmax_s(const StagGraph* csc, const float* el, int64_t el_sample_stride,
+                             const float* er, int64_t er_sample_stride, int32_t H, int32_t S,
+                             const StagNoise* noise, float slope, float* a, void* ws, size_t ws_bytes, void* stream);
+STAG_API int stag_attention_softmax_s_bwd(const StagGraph* csc, const float* el, int64_t el_sample_stride,
+                                 const float* er, int64_t er_sample_stride, int32_t H, int32_t S,
+                                 const StagNoise* noise, float slope, const float* a, const float* da,
+                                 float* dpre, float* d_er, float* dparam0, float* dparam1, float* dw_external,
+                                 void* ws, size_t ws_bytes, void* stream);
+
 /* Likelihood epilogue (stag/models.py:69-72, stag/likelihoods.py:13-38): for each of the S Monte-Carlo outputs
  *   nll_out[s] = mean over the masked nodes of -log_prob(probs[s], y)
  * kind 0: Categorical(probs=.) -- probs renormalised, clamped to [eps, 1-eps], log, gathered at y (int64 [N]);

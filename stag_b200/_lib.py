@@ -90,6 +90,10 @@ SIGNATURES = {
     "stag_edge_softmax_bwd": (_I, [_GP, _V, _V, _I32, _V, _V]),
     "stag_attention_softmax": (_I, [_GP, _V, _V, _V, ctypes.c_float, _I32, _V, _V]),
     "stag_attention_softmax_bwd": (_I, [_GP, _V, _V, _V, ctypes.c_float, _I32, _V, _V, _V, _V, _V, _V]),
+    "stag_attention_workspace_bytes": (_SZ, [_GP, _I32, _I32]),
+    "stag_attention_softmax_s": (_I, [_GP, _V, _I64, _V, _I64, _I32, _I32, _NP, ctypes.c_float, _V, _V, _SZ, _V]),
+    "stag_attention_softmax_s_bwd": (_I, [_GP, _V, _I64, _V, _I64, _I32, _I32, _NP, ctypes.c_float, _V, _V, _V, _V,
+                                          _V, _V, _V, _V, _SZ, _V]),
     "stag_nll_workspace_bytes": (_SZ, [_I64, _I32]),
     "stag_nll": (_I, [_V, _I64, _I64, _I64, _I32, _I32, _I, _V, _I64, _V, _V, _V, _V, _V, _SZ, _V]),
     "stag_gemm_workspace_bytes": (_SZ, [_I64, _I32, _I32]),

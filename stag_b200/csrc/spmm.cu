@@ -32,6 +32,7 @@
 #include <stdlib.h>
 #include "common.cuh"
 #include "noise.cuh"
+#include "param_finalize.cuh"
 
 #ifndef STAG_PACK2
 #define STAG_PACK2 1  // packed fp32 (FFMA2 / FMUL2) Box-Muller + accumulate in agg_stream_kernel
@@ -1442,46 +1443,6 @@ __global__ void hub_finalize_kernel(const AggParams p, int grads) {
   }
   if (p.rscale) acc *= p.rscale[row];
   if (p.out) p.out[(int64_t)s * p.out_ss + (int64_t)row * p.ldo + c] = acc;
-}
-
-// Reduce per-CTA parameter-gradient partials in CTA order (deterministic).
-__global__ void param_finalize_kernel(const float* __restrict__ partial, int ncta, int D8, int D, int scalar,
-                                      float* __restrict__ dp0, float* __restrict__ dp1) {
-  __shared__ float red[2][256];
-  const int tid = threadIdx.x;
-  if (!scalar) {
-    const int c = blockIdx.x * blockDim.x + tid;
-    if (c >= D) return;
-    float a = 0.f, b = 0.f;
-    for (int k = 0; k < ncta; ++k) {
-      a += partial[(size_t)k * 2 * D8 + c];
-      b += partial[(size_t)k * 2 * D8 + D8 + c];
-    }
-    dp0[c] = a;
-    dp1[c] = b;
-  } else {
-    float a = 0.f, b = 0.f;
-    for (int c = tid; c < D; c += blockDim.x) {
-      for (int k = 0; k < ncta; ++k) {
-        a += partial[(size_t)k * 2 * D8 + c];
-        b += partial[(size_t)k * 2 * D8 + D8 + c];
-      }
-    }
-    red[0][tid] = a;
-    red[1][tid] = b;
-    __syncthreads();
-    for (int o = blockDim.x >> 1; o > 0; o >>= 1) {
-      if (tid < o) {
-        red[0][tid] += red[0][tid + o];
-        red[1][tid] += red[1][tid + o];
-      }
-      __syncthreads();
-    }
-    if (tid == 0) {
-      dp0[0] = red[0][0];
-      dp1[0] = red[1][0];
-    }
-  }
 }
 
 // Per-edge parameter gradients (EDGE / EDGE_CHANNEL shapes: the [E,1] / [E,K] outputs of AmortizedDistribution,

@@ -5,9 +5,9 @@ What changed underneath: the reference draws an ``[E,K]`` noise tensor with
 ``q_a.expand([E,K]).rsample()`` (stag/layers.py:115-129), optionally applies relu and
 ``_in_norm`` (:98-105, :8-36) and hands the tensor to ``base_layer.forward(edge_weight=)``
 (:109-113).  Here ``forward`` hands fused-capable base layers (everything in
-``stag_b200.zoo`` except GAT) a lazy :class:`~stag_b200.ops.NoiseSpec` in the same
-``edge_weight=`` slot; the CUDA kernel generates, transforms, normalises and consumes
-the noise in one pass and regenerates it in the backward.  Base layers that are not
+``stag_b200.zoo``) a lazy :class:`~stag_b200.ops.NoiseSpec` in the same
+``edge_weight=`` slot (GAT included: its attention kernel draws the logit noise); the CUDA kernel generates,
+transforms, normalises and consumes the noise in one pass and regenerates it in the backward.  Base layers that are not
 fused, and the vi+norm combination, receive a real tensor emitted from the same Philox
 stream (``stag_noise_emit``), so both routes see identical noise.
 """

@@ -58,10 +58,12 @@ class StagModel(torch.nn.Module):
             if isinstance(layer, StagLayer):
                 if not getattr(layer.base_layer, "accepts_noise_spec", False):
                     return False
-                # a base layer must say that it takes [S,N,D] features with a sample-batched NoiseSpec
-                # (GatedGCN takes a NoiseSpec but runs its BatchNorm per pass: sequential passes, as the reference)
+                # a base layer must say that it takes [S,N,D] features with a sample-batched NoiseSpec: GCN, SAGE, GIN and
+                # GAT do (GAT's attention kernel draws the logit noise of all S samples in one launch); GatedGCN takes a
+                # NoiseSpec but runs its BatchNorm per pass: sequential passes, as the reference
                 if not getattr(layer.base_layer, "accepts_sample_batch", False):
                     return False
+                # an amortised posterior conditions on the [N,D] features of one pass, not on [S,N,D] ones
                 if layer.q_a.__class__.__name__ == "AmortizedDistribution":
                     return False
                 if layer.q_a.fused_parameters() is None or (layer.norm and layer.vi):

@@ -622,11 +622,13 @@ def _aggregate_max(g, feat, edge_weight, S, shared):
 
 
 class _HeadsAggregate(torch.autograd.Function):
-    """out[v, k, :] = sum over the in-edges e = (u, v) of a[e, k] * ft[u, k, :]  -- the weighted aggregation of a
-    multi-head attention layer (GATConv's ``u_mul_e('ft', 'a') -> sum``).  One launch per head on the per-edge-weight
-    kernel, each reading its F columns of ``ft`` IN PLACE (row stride H F) and writing its F columns of ``out`` in
-    place: no ``[E, H F]`` expansion of the attention, no per-head copies.  Backward: per head the transposed pass
-    (d ft) and the SDDMM (d a) in one ``stag_spmm_bwd`` call."""
+    """out[(s,) v, k, :] = sum over the in-edges e = (u, v) of a[(s,) e, k] * ft[(s,) u, k, :]  -- the weighted aggregation
+    of a multi-head attention layer (GATConv's ``u_mul_e('ft', 'a') -> sum``).  One launch per head on the per-edge-weight
+    kernel, covering every Monte-Carlo sample, each reading its F columns of ``ft`` IN PLACE (row stride H F; sample
+    stride 0 when ``ft`` is shared) and writing its F columns of ``out`` in place: no ``[E, H*F]`` expansion of the
+    attention, no per-head copies.  The attention is permuted to ``[H, S, E]`` so that the weights of head k are one
+    ``[S, E, 1]`` external tensor.  Backward: per head the transposed pass (d ft) and the SDDMM (d a) in one
+    ``stag_spmm_bwd`` call."""
 
     @staticmethod
     def forward(ctx, ft, a, graph):
@@ -636,54 +638,71 @@ class _HeadsAggregate(torch.autograd.Function):
         lib = _lib.load()
         N, NS, E = st.num_nodes, st.num_src, st.num_edges
         H, F = ft.shape[-2], ft.shape[-1]
-        x = _c(ft.to(torch.float32)).reshape(NS, H * F)
-        at = a.detach().to(torch.float32).t().contiguous()               # [H, E]: the weights of a head are one row
-        out = torch.empty((N, H * F), dtype=torch.float32, device=dev)
+        batched = a.dim() == 3
+        S = a.shape[0] if batched else 1
+        shared = ft.dim() == 3
+        x = _c(ft.to(torch.float32)).reshape(-1, NS, H * F)
+        at = a.detach().to(torch.float32).reshape(S, E, H).permute(2, 0, 1).contiguous()   # [H, S, E]: a head's weights
+        xs = 0 if shared else NS * H * F
+        out = torch.empty((S, N, H * F), dtype=torch.float32, device=dev)
         with _on_device(dev):
             csc, _ = st.csx(True)
-            ws = _workspace(st, lib, csc, True, F, 1)
+            ws = _workspace(st, lib, csc, True, F, S)
             for k in range(H):
                 nz = _fill_noise(None, _lib.NOISE_EXTERNAL, 1, None, None, at[k], False, False, 0, 0, 0, _lib.PARAM_SCALAR)
                 _lib.check(lib.stag_spmm_fwd(
-                    ctypes.byref(csc), x.data_ptr() + 4 * k * F, H * F, 0, F, 1, ctypes.byref(nz), 0, 0,
+                    ctypes.byref(csc), x.data_ptr() + 4 * k * F, H * F, xs, F, S, ctypes.byref(nz), 0, 0,
                     out.data_ptr() + 4 * k * F, H * F, N * H * F, 0, ws.data_ptr(), ws.numel(), _stream(dev)))
-        ctx.graph, ctx.dims = graph, (N, NS, E, H, F)
+        ctx.graph, ctx.dims, ctx.flags = graph, (N, NS, E, H, F, S), (batched, shared)
         ctx.save_for_backward(x, at)
-        return out.reshape(N, H, F)
+        return out.reshape(S, N, H, F) if batched else out.reshape(N, H, F)
 
     @staticmethod
     def backward(ctx, gout):
         x, at = ctx.saved_tensors
-        N, NS, E, H, F = ctx.dims
+        N, NS, E, H, F, S = ctx.dims
+        batched, shared = ctx.flags
         st = ctx.graph._s
         lib = _lib.load()
         dev = gout.device
-        g2 = gout.to(torch.float32).contiguous().reshape(N, H * F)
+        g2 = gout.to(torch.float32).contiguous().reshape(S, N, H * F)
+        xs = 0 if shared else NS * H * F
         need_dx, need_da = ctx.needs_input_grad[0], ctx.needs_input_grad[1]
-        dx = torch.empty((NS, H * F), dtype=torch.float32, device=dev) if need_dx else None
-        dat = torch.empty((H, E), dtype=torch.float32, device=dev) if need_da else None
+        dx = torch.empty((S, NS, H * F), dtype=torch.float32, device=dev) if need_dx else None
+        dat = torch.empty((H, S, E), dtype=torch.float32, device=dev) if need_da else None
         with _on_device(dev):
             csr, _ = st.csx(False)
-            ws = _workspace(st, lib, csr, False, F, 1)
+            ws = _workspace(st, lib, csr, False, F, S)
             for k in range(H):
                 nz = _fill_noise(None, _lib.NOISE_EXTERNAL, 1, None, None, at[k], False, False, 0, 0, 0, _lib.PARAM_SCALAR)
                 if need_da:
                     _lib.check(lib.stag_spmm_bwd(
-                        ctypes.byref(csr), x.data_ptr() + 4 * k * F, H * F, 0, g2.data_ptr() + 4 * k * F, H * F, N * H * F,
-                        F, 1, ctypes.byref(nz), 0, 0, 0 if dx is None else dx.data_ptr() + 4 * k * F, H * F, NS * H * F,
-                        0, 0, dat[k].data_ptr(), ws.data_ptr(), ws.numel(), _stream(dev)))
+                        ctypes.byref(csr), x.data_ptr() + 4 * k * F, H * F, xs, g2.data_ptr() + 4 * k * F, H * F,
+                        N * H * F, F, S, ctypes.byref(nz), 0, 0, 0 if dx is None else dx.data_ptr() + 4 * k * F, H * F,
+                        NS * H * F, 0, 0, dat[k].data_ptr(), ws.data_ptr(), ws.numel(), _stream(dev)))
                 elif need_dx:
                     _lib.check(lib.stag_spmm_fwd(
-                        ctypes.byref(csr), g2.data_ptr() + 4 * k * F, H * F, 0, F, 1, ctypes.byref(nz), 0, 0,
+                        ctypes.byref(csr), g2.data_ptr() + 4 * k * F, H * F, N * H * F, F, S, ctypes.byref(nz), 0, 0,
                         dx.data_ptr() + 4 * k * F, H * F, NS * H * F, 0, ws.data_ptr(), ws.numel(), _stream(dev)))
-        return (None if dx is None else dx.reshape(NS, H, F)), (None if dat is None else dat.t()), None
+        gft = gat = None
+        if dx is not None:
+            gft = (dx.sum(0) if shared and batched else dx).reshape((NS, H, F) if shared else (S, NS, H, F))
+        if dat is not None:
+            gat = dat.permute(1, 2, 0) if batched else dat[:, 0].t()
+        return gft, gat, None
 
 
 def heads_aggregate(graph, ft, a):
-    """Per-head weighted aggregation ``[N_src, H, F], [E, H] -> [N, H, F]`` (see :class:`_HeadsAggregate`)."""
+    """Per-head weighted aggregation ``[N_src, H, F], [E, H] -> [N, H, F]``, or over S Monte-Carlo samples
+    ``[S, N_src, H, F]`` (or a shared ``[N_src, H, F]``), ``[S, E, H] -> [S, N, H, F]`` (see :class:`_HeadsAggregate`)."""
     g = as_graph(graph)
-    if ft.dim() != 3 or a.dim() != 2 or a.shape[1] != ft.shape[1] or a.shape[0] != g.number_of_edges():
-        raise ValueError("heads_aggregate: feat [N,H,F] and attention [E,H] expected, got %s and %s"
+    ok = ft.dim() in (3, 4) and a.dim() in (2, 3) and a.shape[-1] == ft.shape[-2] and a.shape[-2] == g.number_of_edges()
+    if ok and a.dim() == 2:
+        ok = ft.dim() == 3
+    elif ok:
+        ok = ft.dim() == 3 or ft.shape[0] == a.shape[0]
+    if not ok:
+        raise ValueError("heads_aggregate: feat [N,H,F] or [S,N,H,F] and attention [E,H] or [S,E,H] expected, got %s and %s"
                          % (tuple(ft.shape), tuple(a.shape)))
     return _HeadsAggregate.apply(ft, a, g)
 
@@ -752,77 +771,189 @@ class _EdgeSoftmax(torch.autograd.Function):
 
 
 class _AttentionSoftmax(torch.autograd.Function):
-    """a[e,h] = softmax over the in-edges of v_e of  w[e,h] * leaky_relu(el[u_e,h] + er[v_e,h])  -- GAT's attention
-    (stag/zoo/gat.py:113-122) without the [E,H] logits and their autograd graph (stag_attention_softmax).  Backward: one
-    pass over the CSC rows gives d w, d er and the per-edge d(el + er); d el is their sum per SOURCE node, taken by the
-    aggregation kernel on the CSR (edge values as external weights of a ones operand).  No atomics: deterministic."""
+    """a[(s,) e, h] = softmax over the in-edges of v_e of  w[(s,) e, h] * leaky_relu(el[(s,) u_e, h] + er[(s,) v_e, h])  --
+    GAT's attention (stag/zoo/gat.py:113-122) without the [E,H] logits and their autograd graph.  The noise w is none, an
+    external tensor, or drawn inside the kernel from a NoiseSpec (S samples per launch, stag_attention_softmax_s);
+    unbatched calls without a spec take the S = 1 entry points (stag_attention_softmax).  Backward: one pass over the CSC
+    rows gives d er, the per-edge d(el + er), d w (external) or the parameter gradients (generated); d el is the sum per
+    SOURCE node of the per-edge values, taken by the aggregation kernel on the CSR (edge values as external weights of a
+    ones operand).  No atomics: deterministic."""
 
     @staticmethod
-    def forward(ctx, el, er, w, g, slope):
+    def forward(ctx, el, er, p0, p1, ext, cfg):
         _require_cuda(el, "el")
         lib = _lib.load()
         dev = el.device
-        st = g._s
-        E, H = st.num_edges, el.shape[-1]
-        elc, erc = el.detach().to(torch.float32).contiguous(), er.detach().to(torch.float32).contiguous()
-        wc = None if w is None else w.detach().to(torch.float32).contiguous()
-        a = torch.empty((E, H), dtype=torch.float32, device=dev)
+        st = cfg["graph"]._s
+        E, H, S = st.num_edges, el.shape[-1], cfg["S"]
+        elc, erc = _c(el), _c(er)
+        p0c, p1c, extc = _c(p0), _c(p1), _c(ext)
+        a = torch.empty((S, E, H), dtype=torch.float32, device=dev)
         with _on_device(dev):
             csc, _ = st.csx(True)
-            _lib.check(lib.stag_attention_softmax(ctypes.byref(csc), elc.data_ptr(), erc.data_ptr(), _ptr(wc), float(slope), H,
-                                                  a.data_ptr(), _stream(dev)))
-        ctx.g, ctx.slope = g, float(slope)
-        ctx.save_for_backward(elc, erc, wc, a)
+            if cfg["legacy"]:
+                _lib.check(lib.stag_attention_softmax(ctypes.byref(csc), elc.data_ptr(), erc.data_ptr(), _ptr(extc),
+                                                      cfg["slope"], H, a.data_ptr(), _stream(dev)))
+            else:
+                nz = _attention_noise(cfg, p0c, p1c, extc)
+                _lib.check(lib.stag_attention_softmax_s(
+                    ctypes.byref(csc), elc.data_ptr(), 0 if cfg["el_shared"] else st.num_src * H, erc.data_ptr(),
+                    0 if cfg["er_shared"] else st.num_nodes * H, H, S, ctypes.byref(nz), cfg["slope"], a.data_ptr(),
+                    0, 0, _stream(dev)))
+        ctx.cfg = cfg
+        ctx.param_shapes = (None if p0 is None else p0.shape, None if p1 is None else p1.shape)
+        ctx.ext_shape = None if ext is None else ext.shape
+        ctx.save_for_backward(elc, erc, p0c, p1c, extc, a)
         return a
 
     @staticmethod
     def backward(ctx, da):
-        elc, erc, wc, a = ctx.saved_tensors
+        elc, erc, p0c, p1c, extc, a = ctx.saved_tensors
+        cfg = ctx.cfg
         lib = _lib.load()
         dev = a.device
-        st = ctx.g._s
-        E, H = a.shape
-        d_er = torch.zeros_like(erc)
-        d_el = torch.zeros_like(elc)
-        dw = None
+        st = cfg["graph"]._s
+        S, E, H = a.shape
+        N, NS = st.num_nodes, st.num_src
+        need_dp = (ctx.needs_input_grad[2] or ctx.needs_input_grad[3]) and cfg["kind"] in (
+            _lib.NOISE_NORMAL, _lib.NOISE_UNIFORM)
+        need_dext = ctx.needs_input_grad[4] and cfg["kind"] == _lib.NOISE_EXTERNAL
+        d_er = torch.zeros((S, N, H), dtype=torch.float32, device=dev)
+        d_el = torch.zeros((S, NS, H), dtype=torch.float32, device=dev)
+        dext = torch.zeros_like(a) if need_dext else None
+        dp0 = dp1 = None
+        if need_dp:
+            n = {_lib.PARAM_SCALAR: 1, _lib.PARAM_CHANNEL: H, _lib.PARAM_EDGE: E,
+                 _lib.PARAM_EDGE_CHANNEL: E * H}[cfg["param_shape"]]
+            dp0 = torch.zeros(n, dtype=torch.float32, device=dev)
+            dp1 = torch.zeros(n, dtype=torch.float32, device=dev)
         if E:
             da = da.to(torch.float32).contiguous()
-            dw = torch.empty_like(a) if (wc is not None and ctx.needs_input_grad[2]) else None
             dpre = torch.empty_like(a)
             with _on_device(dev):
                 csc, _ = st.csx(True)
-                _lib.check(lib.stag_attention_softmax_bwd(
-                    ctypes.byref(csc), elc.data_ptr(), erc.data_ptr(), _ptr(wc), ctx.slope, H, a.data_ptr(), da.data_ptr(),
-                    _ptr(dw), dpre.data_ptr(), d_er.data_ptr(), _stream(dev)))
+                if cfg["legacy"]:
+                    _lib.check(lib.stag_attention_softmax_bwd(
+                        ctypes.byref(csc), elc.data_ptr(), erc.data_ptr(), _ptr(extc), cfg["slope"], H, a.data_ptr(),
+                        da.data_ptr(), _ptr(dext), dpre.data_ptr(), d_er.data_ptr(), _stream(dev)))
+                else:
+                    ws = _attention_workspace(st, lib, csc, H, S)
+                    nz = _attention_noise(cfg, p0c, p1c, extc)
+                    _lib.check(lib.stag_attention_softmax_s_bwd(
+                        ctypes.byref(csc), elc.data_ptr(), 0 if cfg["el_shared"] else NS * H, erc.data_ptr(),
+                        0 if cfg["er_shared"] else N * H, H, S, ctypes.byref(nz), cfg["slope"], a.data_ptr(),
+                        da.data_ptr(), dpre.data_ptr(), d_er.data_ptr(), _ptr(dp0), _ptr(dp1), _ptr(dext),
+                        ws.data_ptr(), ws.numel(), _stream(dev)))
                 if ctx.needs_input_grad[0]:
-                    # d el[u,h] = sum over the out-edges of u of dpre[e,h]: the aggregation kernel on the CSR, a ones operand
-                    # gathered per destination, the edge values as external per-channel weights
+                    # d el[s,u,h] = sum over the out-edges of u of dpre[s,e,h]: the aggregation kernel on the CSR, a ones
+                    # operand gathered per destination (shared by the samples), the edge values as external weights
                     csr, _ = st.csx(False)
-                    ws = _workspace(st, lib, csr, False, H, 1)
-                    ones = torch.ones((st.num_nodes, H), dtype=torch.float32, device=dev)
+                    ws = _workspace(st, lib, csr, False, H, S)
+                    ones = torch.ones((N, H), dtype=torch.float32, device=dev)
                     nz = _fill_noise(None, _lib.NOISE_EXTERNAL, H, None, None, dpre, False, False, 0, 0, 0, _lib.PARAM_SCALAR)
                     _lib.check(lib.stag_spmm_fwd(
-                        ctypes.byref(csr), ones.data_ptr(), H, 0, H, 1, ctypes.byref(nz), 0, 0, d_el.data_ptr(), H,
-                        st.num_src * H, 0, ws.data_ptr(), ws.numel(), _stream(dev)))
-        elif wc is not None and ctx.needs_input_grad[2]:
-            dw = torch.zeros_like(a)
-        return d_el, d_er, dw, None, None
+                        ctypes.byref(csr), ones.data_ptr(), H, 0, H, S, ctypes.byref(nz), 0, 0, d_el.data_ptr(), H,
+                        NS * H, 0, ws.data_ptr(), ws.numel(), _stream(dev)))
+        gel = d_el.sum(0) if cfg["el_shared"] else d_el
+        ger = d_er.sum(0) if cfg["er_shared"] else d_er
+        gp0 = gp1 = gext = None
+        if need_dp:
+            s0, s1 = ctx.param_shapes
+            if ctx.needs_input_grad[2]:
+                gp0 = dp0.reshape(s0) if dp0.numel() == max(1, _numel(s0)) else dp0.reshape(-1).sum_to_size(s0)
+            if ctx.needs_input_grad[3] and s1 is not None:
+                gp1 = dp1.reshape(s1) if dp1.numel() == max(1, _numel(s1)) else dp1.reshape(-1).sum_to_size(s1)
+        if need_dext:
+            gext = dext.reshape(ctx.ext_shape)
+        return gel.reshape(elc.shape), ger.reshape(erc.shape), gp0, gp1, gext, None
 
 
-def attention_softmax(graph, el, er, edge_weight=None, negative_slope=0.2):
-    """GAT attention ``[E,H]`` from the per-node scores ``el [N_src,H]``, ``er [N,H]`` and optional edge noise ``[E,H]``
-    (see :class:`_AttentionSoftmax`)."""
+def _attention_noise(cfg, p0c, p1c, extc):
+    return _fill_noise(None, cfg["kind"], cfg["K"], p0c, p1c, extc, cfg["relu"], False, cfg["sample_base"], cfg["seed"],
+                       cfg["offset"], cfg["param_shape"])
+
+
+def _attention_workspace(st, lib, csc, H, S):
+    key = ("attention", H, S)
+    cache = st.__dict__.setdefault("_ws_bytes", {})
+    if key not in cache:
+        cache[key] = lib.stag_attention_workspace_bytes(ctypes.byref(csc), H, S)
+    return st.workspace(cache[key])
+
+
+def attention_route(spec):
+    """'fused' when the attention kernel draws the noise of `spec` itself, 'materialized' when the spec goes through its
+    noise tensor (in-norm rescales by a per-row sum the kernel does not take; the tensor-core generator works on
+    128-channel groups, not one channel per head)."""
+    if spec.in_norm or spec.lib_kind == _lib.NOISE_NORMAL_HADAMARD:
+        return "materialized"
+    return "fused"
+
+
+def attention_softmax(graph, el, er, edge_weight=None, negative_slope=0.2, n_samples=None):
+    """GAT attention from the per-node scores ``el [N_src,H]``, ``er [N,H]`` and the logit noise ``edge_weight``: ``None``,
+    a tensor ``[E,H]`` / ``[E,1]`` / ``[E]`` (or ``[S,E,H]``), or a :class:`NoiseSpec` with ``K == H`` drawn inside the
+    kernel.  Returns ``[E,H]``, or ``[S,E,H]`` over S Monte-Carlo samples: with ``n_samples=S``, per-sample scores
+    ``[S,N,H]``, ``[S,E,H]`` weights or a sample-batched spec; ``[N,H]`` scores are then shared by the samples (see
+    :class:`_AttentionSoftmax`)."""
     g = as_graph(graph)
-    E = g.number_of_edges()
-    if el.dim() != 2 or er.dim() != 2 or el.shape[1] != er.shape[1]:
-        raise ValueError("attention_softmax: el [N_src,H] and er [N,H] expected, got %s and %s" % (tuple(el.shape), tuple(er.shape)))
-    w = edge_weight
-    if w is not None:
-        w = w.unsqueeze(-1) if w.dim() == 1 else w.flatten(1)
-        if w.shape[0] != E or w.shape[1] not in (1, el.shape[1]):
-            raise ValueError("attention_softmax: edge_weight must be [E,H] or [E,1], got %s" % (tuple(edge_weight.shape),))
-        w = w.expand(E, el.shape[1])
-    return _AttentionSoftmax.apply(el, er, w, g, negative_slope)
+    st = g._s
+    E = st.num_edges
+    if el.dim() not in (2, 3) or er.dim() not in (2, 3) or el.shape[-1] != er.shape[-1]:
+        raise ValueError("attention_softmax: el [(S,)N_src,H] and er [(S,)N,H] expected, got %s and %s"
+                         % (tuple(el.shape), tuple(er.shape)))
+    H = el.shape[-1]
+    if el.shape[-2] != st.num_src or er.shape[-2] != st.num_nodes:
+        raise ValueError("attention_softmax: el has %d rows and er %d, graph has %d source and %d destination nodes"
+                         % (el.shape[-2], er.shape[-2], st.num_src, st.num_nodes))
+    spec = edge_weight if isinstance(edge_weight, NoiseSpec) else None
+    S = None if n_samples is None else int(n_samples)
+    for t in (el, er) + ((edge_weight,) if (edge_weight is not None and spec is None and edge_weight.dim() == 3) else ()):
+        if t.dim() == 3:
+            if S is not None and t.shape[0] != S:
+                raise ValueError("attention_softmax: inputs disagree on the number of samples (%d and %d)" % (S, t.shape[0]))
+            S = t.shape[0]
+    if S is None and spec is not None and spec.batched:
+        S = spec.n_samples
+    batched = S is not None
+    S = 1 if S is None else S
+    if spec is not None:
+        if spec.num_edges != E:
+            raise ValueError("noise spec was made for %d edges, graph has %d" % (spec.num_edges, E))
+        if spec.K != H:
+            raise ValueError("attention noise width K=%d must equal the number of heads H=%d" % (spec.K, H))
+        if attention_route(spec) == "materialized":
+            w = spec.materialize(n_samples=S)                                       # [S,E,H], relu applied
+            if spec.in_norm:
+                from .layers import _in_norm
+                w = torch.stack([_in_norm(g, w[s]) for s in range(S)])
+            a = attention_softmax(g, el, er, w, negative_slope, n_samples=S)
+            return a if batched else a[0]
+    cfg = {"graph": g, "S": S, "el_shared": el.dim() == 2, "er_shared": er.dim() == 2, "slope": float(negative_slope),
+           "kind": _lib.NOISE_NONE, "K": H, "relu": False, "sample_base": 0, "seed": 0, "offset": 0,
+           "param_shape": _lib.PARAM_SCALAR, "legacy": False}
+    p0 = p1 = ext = None
+    if spec is not None:
+        cfg.update(kind=spec.lib_kind, relu=spec.relu, sample_base=spec.sample_base, seed=spec.seed, offset=spec.offset,
+                   param_shape=spec.param_shape)
+        p0, p1 = spec.p0, spec.p1
+    elif edge_weight is not None:
+        w = edge_weight
+        _require_cuda(w, "edge_weight")
+        if w.dim() == 3:
+            if w.shape[1] != E or w.shape[2] not in (1, H):
+                raise ValueError("attention_softmax: edge_weight must be [E,H], [E,1] or [S,E,H], got %s"
+                                 % (tuple(edge_weight.shape),))
+        else:
+            w = w.unsqueeze(-1) if w.dim() == 1 else w.flatten(1)
+            if w.shape[0] != E or w.shape[1] not in (1, H):
+                raise ValueError("attention_softmax: edge_weight must be [E,H] or [E,1], got %s" % (tuple(edge_weight.shape),))
+            w = w.unsqueeze(0)
+        ext = w.expand(S, E, H)
+        cfg["kind"] = _lib.NOISE_EXTERNAL
+    cfg["legacy"] = not batched and spec is None
+    a = _AttentionSoftmax.apply(el, er, p0, p1, ext, cfg)
+    return a if batched else a[0]
 
 
 def edge_softmax(graph, logits):

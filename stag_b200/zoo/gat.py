@@ -2,11 +2,13 @@
 The noise ``[E,H]`` multiplies the pre-softmax logits (:117-119).  Attention: the logits
 ``edge_weight * leaky_relu(el[u] + er[v])`` are computed INSIDE the segmented softmax over the in-edges of each node
 (``stag_attention_softmax``, forward and a deterministic backward, csrc/edge_softmax.cu: no ``[E,H]`` logits, no atomics).
+With a :class:`~stag_b200.ops.NoiseSpec` in ``edge_weight=`` (``accepts_noise_spec``) the kernel draws the logit noise
+itself and runs S Monte-Carlo samples per launch (``accepts_sample_batch``: ``[S,N,D]`` features, or shared ``[N,D]``
+ones with a sample-batched spec); in-norm specs go through the materialised noise tensor.
 The weighted aggregation ``update_all(u_mul_e('ft','a'), sum)`` (:125-126) runs on ``stag_spmm_fwd`` with the attention as
-external weights: all heads in one launch with expanded ``[E, H*F]`` weights on small (launch-bound) graphs (<= 4 MB),
-else ``ops.heads_aggregate`` -- one launch per head, every head reading / writing its F columns in place.
-``accepts_noise_spec`` is False: the noise multiplies the LOGITS, not the messages, so ``StagLayer`` hands this
-layer a tensor emitted from the library's Philox stream (``stag_noise_emit``, K = num_heads).
+external weights: all heads in one launch with expanded ``[(S,) E, H*F]`` weights on small (launch-bound) graphs
+(<= 4 MB), else ``ops.heads_aggregate`` -- one launch per head over every sample, each head reading / writing its F
+columns in place.
 """
 import torch
 from torch import nn
@@ -16,7 +18,8 @@ from ..graph import as_graph
 
 
 class GAT(nn.Module):
-    accepts_noise_spec = False
+    accepts_noise_spec = True
+    accepts_sample_batch = True
 
     def __init__(self, in_feats, out_feats, last=False, num_heads=4, feat_drop=0.0, attn_drop=0.0,
                  negative_slope=0.2, residual=False, activation=None, allow_zero_in_degree=False, bias=True):
@@ -59,27 +62,35 @@ class GAT(nn.Module):
 
     def forward(self, graph, feat, get_attention=False, edge_weight=None):
         g = as_graph(graph)
-        src, dst = g.edges()
-        N, H, F = g.number_of_nodes(), self._num_heads, self._out_feats
+        H, F = self._num_heads, self._out_feats
+        E = g.number_of_edges()
+        # S Monte-Carlo samples: [S,N,D] features, or shared [N,D] ones with a sample-batched NoiseSpec
+        S = feat.shape[0] if feat.dim() == 3 else ops.spec_samples(edge_weight, feat)
+        if S is not None and feat.dim() == 2 and self.training and self.feat_drop.p > 0:
+            # one dropout mask per sample, as S sequential passes draw them
+            feat = feat.unsqueeze(0).expand((S,) + tuple(feat.shape))
         h = self.feat_drop(feat)
-        ft = self.fc(h).view(N, H, F)
+        ft = self.fc(h).view(tuple(h.shape[:-1]) + (H, F))                        # [(S,) N, H, F]
         el = (ft * self.attn_l).sum(dim=-1)
         er = (ft * self.attn_r).sum(dim=-1)
         # attention: softmax over the in-edges of  edge_weight * leaky_relu(el[u] + er[v])  in one fused pass per direction
-        # (stag_attention_softmax: the [E,H] logits and their autograd graph never exist)
-        a = self.attn_drop(ops.attention_softmax(g, el, er, edge_weight, self.leaky_relu.negative_slope))   # [E,H]
-        if a.shape[0] * H * F * 4 <= (4 << 20):
+        # (stag_attention_softmax: the [E,H] logits and their autograd graph never exist; a NoiseSpec is drawn inside)
+        a = self.attn_drop(ops.attention_softmax(g, el, er, edge_weight, self.leaky_relu.negative_slope,
+                                                 n_samples=S))                    # [(S,) E, H]
+        lead = tuple(ft.shape[:-3])                                                # (S,) for per-sample features
+        if (1 if S is None else S) * E * H * F * 4 <= (4 << 20):
             # small graphs are launch-bound: ONE fused launch over the H*F channels, the attention of head k expanded to the
-            # weight of channels k*F .. (k+1)*F - 1 (external per-channel weights [E, H*F], at most 4 MB; autograd sums the
-            # SDDMM gradient back over the F channels of a head)
-            aw = a.unsqueeze(-1).expand(a.shape[0], H, F).reshape(a.shape[0], H * F)
-            rst = ops.stochastic_aggregate(g, ft.reshape(N, H * F), aw).view(N, H, F)
+            # weight of channels k*F .. (k+1)*F - 1 (external per-channel weights [(S,) E, H*F], at most 4 MB; autograd sums
+            # the SDDMM gradient back over the F channels of a head)
+            aw = a.unsqueeze(-1).expand(tuple(a.shape) + (F,)).reshape(tuple(a.shape[:-1]) + (H * F,))
+            rst = ops.stochastic_aggregate(g, ft.reshape(lead + (ft.shape[-3], H * F)), aw, n_samples=S)
+            rst = rst.view(tuple(rst.shape[:-1]) + (H, F))
         else:
             # one launch per head on the per-edge-weight kernel, every head reading / writing its F columns in place (row
             # stride H*F): no [E, H*F] expansion, no per-head copies
             rst = ops.heads_aggregate(g, ft, a)
         if self.res_fc is not None:
-            rst = rst + self.res_fc(h).view(N, -1, F)
+            rst = rst + self.res_fc(h).view(tuple(h.shape[:-1]) + (-1, F))
         if self.bias is not None:
             rst = rst + self.bias.view(1, H, F)
         rst = rst.mean(-2) if self.last else rst.flatten(-2, -1)
