@@ -96,7 +96,9 @@ typedef struct StagGraph {
   const int32_t* hub_rows;     /* [num_hubs]   row ids, increasing                */
   const int32_t* hub_seg_ptr;  /* [num_hubs+1] first global segment of each hub   */
   /* processing order of the rows (decreasing stored-edge count) so that rows sharing a warp have
-   * equal trip counts; NULL = natural order.  Results do not depend on it. */
+   * equal trip counts; NULL = natural order.  Results do not depend on it, except for the last bits of the summed
+   * SCALAR / CHANNEL parameter gradients of stag_spmm_bwd on the row-per-group path (per-CTA partials are added in
+   * the order the rows are visited). */
   const int32_t* row_order;    /* [num_rows] or NULL                              */
   /* stream items: consecutive row ranges {row0, row1, e0, e1} holding about 64 stored edges each
    * (e1 = -1: placeholder of a hub row), by decreasing edge count: the unit of work of the
