@@ -329,6 +329,27 @@ STAG_API int stag_nll(const float* probs, int64_t ld, int64_t sample_stride, int
              int kind, const void* y, int64_t ldy, const uint8_t* mask, float* nll_out, float* count_out,
              float* dprobs, void* ws, size_t ws_bytes, void* stream);
 
+/* Monte-Carlo predictive statistics in bounded memory.  probs[s] (s < S) is the raw [N,C] output of one Monte-Carlo
+ * sample (row stride ld, sample stride sample_stride, which may be 0).  acc_sum [N,C] (contiguous) and acc_ent [N] are
+ * float64, caller-owned and caller-zeroed; stag_mc_accumulate ADDS to them:
+ *   acc_sum += p_s,   acc_ent += H(p_s)
+ * in sample order, one row per warp, no atomics: calls over consecutive chunks of samples give the same bits whatever
+ * the chunk sizes, and two chunked passes over disjoint sample ranges can be summed (sample sharding).
+ * kind 0: H = Categorical(probs=.).entropy() = -sum_c q_c log(clamp(q_c, eps, 1-eps)), q = p / sum(p);
+ * kind 1: H = sum over the C labels of Bernoulli(probs=.).entropy(); eps = torch.finfo(float32).eps.
+ * A row that sums to zero or holds a NaN gives NaN, as in torch.  C <= 1024 (STAG_EUNSUPPORTED above).
+ * stag_mc_finalize, with S_total the number of samples accumulated:
+ *   mean = acc_sum / S_total ([N,C] contiguous), pred_entropy = H(mean), exp_entropy = acc_ent / S_total,
+ *   mutual_info = pred_entropy - exp_entropy,
+ *   loglik (optional, with y) = Categorical(probs=mean).log_prob(y), y int64 [N] (NaN outside [0, C)), or the sum over
+ *   the labels of Bernoulli(probs=mean).log_prob(y), y float [N,C] with row stride ldy; y and loglik are both NULL or
+ *   both set. */
+STAG_API int stag_mc_accumulate(const float* probs, int64_t ld, int64_t sample_stride, int64_t N, int32_t C, int32_t S,
+                       int kind, double* acc_sum, double* acc_ent, void* stream);
+STAG_API int stag_mc_finalize(const double* acc_sum, const double* acc_ent, int64_t N, int32_t C, int64_t S_total,
+                     int kind, const void* y, int64_t ldy, float* mean, float* pred_entropy, float* exp_entropy,
+                     float* mutual_info, float* loglik, void* stream);
+
 /* Dense feature transform agg @ W (stag/zoo/gcn.py:97-98) on tcgen05 tensor cores with TMEM
  * accumulators; fp32 in / fp32 out computed as 3xTF32 (fp32-level accuracy), fused epilogue
  *   out[m,n] = act( row_scale[m] * sum_k a[m,k]*w[k,n] + bias[n] ),  act: 0 none, 1 relu.

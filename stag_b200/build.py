@@ -12,7 +12,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT_DIR = os.path.join(HERE, "_C")
 LIB_PATH = os.path.join(OUT_DIR, "libstag_b200.so")
-SOURCES = ["runtime.cu", "csx_build.cu", "spmm.cu", "gemm_tcgen05.cu", "nll.cu", "edge_softmax.cu", "host_api.cu"]
+SOURCES = ["runtime.cu", "csx_build.cu", "spmm.cu", "gemm_tcgen05.cu", "nll.cu", "mc_predictive.cu", "edge_softmax.cu", "host_api.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden",

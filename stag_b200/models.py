@@ -9,10 +9,12 @@ stochastic layer is fused) the S samples travel through the layers together as
 once.  Feature-only layers (BatchNorm / Dropout ...) are still applied per sample, in
 sample order, so their semantics (batch statistics, running averages) are unchanged.
 """
-from typing import List
+from typing import List, NamedTuple, Optional
 
 import torch
+import torch.distributed as dist
 
+from . import ops, parallel, random as _random
 from .layers import StagLayer
 from .likelihoods import Likelihood, CategoricalLikelihood
 from .graph import as_graph
@@ -32,6 +34,45 @@ def nll_contrastive(q_a, graph, feat):
     nll = -q_a.log_prob(torch.tensor(1.0, device=feat.device)) \
         - q_a_negative.log_prob(torch.tensor(0.0, device=feat.device))
     return nll.sum(dim=-1).mean()
+
+
+class Predictive(NamedTuple):
+    """Monte-Carlo predictive of ``n_samples`` stochastic passes, per node: the mean output (what
+    ``forward(..., return_parameters=True)`` returns), the entropy of the predictive distribution (total uncertainty),
+    the mean entropy of the per-sample distributions (aleatoric), their difference (mutual information between the
+    label and the noise: epistemic) and the log-likelihood of the labels under the mean (None without labels)."""
+    mean: torch.Tensor
+    entropy: torch.Tensor
+    expected_entropy: torch.Tensor
+    mutual_information: torch.Tensor
+    log_likelihood: Optional[torch.Tensor]
+    n_samples: int
+
+
+def mc_predictive(chunks, n_samples, kind, y=None, group=None, accumulate=None, finalize=None):
+    """:class:`Predictive` of ``n_samples`` Monte-Carlo outputs, of which ``chunks`` yields this rank's as ``[s,N,C]``
+    tensors in sample order.  Each chunk is added to two float64 accumulators and dropped, so memory does not grow with
+    the number of samples.  With ``group`` the accumulators of the ranks are views of one flat buffer, summed by one
+    all-reduce before the statistics are taken: every rank returns the statistics of all ``n_samples``.
+    ``accumulate`` / ``finalize`` default to the CUDA kernels (:func:`ops.mc_accumulate`, :func:`ops.mc_finalize`)."""
+    accumulate = accumulate or ops.mc_accumulate
+    finalize = finalize or ops.mc_finalize
+    flat = acc_sum = acc_ent = None
+    for out in chunks:
+        if out.dim() != 3:
+            raise ValueError("Monte-Carlo predictive: the model output must be [N, C], got %s per sample"
+                             % (tuple(out.shape[1:]),))
+        if flat is None:
+            N, C = out.shape[1:]
+            flat = torch.zeros(N * C + N, dtype=torch.float64, device=out.device)
+            acc_sum, acc_ent = flat[: N * C].view(N, C), flat[N * C:]
+        accumulate(out, acc_sum, acc_ent, kind)
+        del out   # before the next chunk is computed: only one chunk of outputs is alive at a time
+    if flat is None:
+        raise ValueError("Monte-Carlo predictive: no samples")
+    if group is not None and dist.get_world_size(group) > 1:
+        dist.all_reduce(flat, op=dist.ReduceOp.SUM, group=group)
+    return Predictive(*finalize(acc_sum, acc_ent, n_samples, kind, y), n_samples=int(n_samples))
 
 
 class StagModel(torch.nn.Module):
@@ -106,6 +147,50 @@ class StagModel(torch.nn.Module):
         if return_parameters is True:
             return feat
         return self.likelihood.condition(feat).sample()
+
+    def predictive(self, graph, feat, n_samples, chunk_samples=None, y=None, group=None):
+        """Monte-Carlo predictive of ``n_samples`` stochastic passes with per-node uncertainty (:class:`Predictive`),
+        in memory that does not grow with ``n_samples``: the samples run ``chunk_samples`` at a time (all at once
+        when None) and each chunk's outputs are reduced into float64 accumulators by one kernel and dropped.
+        Models that run their samples as sequential passes (GatedGCN, amortised posteriors) accumulate one pass at a
+        time.  The samples drawn are those of ``forward(n_samples=n_samples)`` from the same Philox state, whatever the
+        chunk size, and the state is left where that call would leave it.  ``y``: labels for the log-likelihood.
+        ``group``: a ``torch.distributed`` group whose ranks shard the samples (``parallel.shard_samples``, common
+        seed); every rank returns the statistics of all ``n_samples``.  No autograd."""
+        kind = getattr(self.likelihood, "fused_kind", None)
+        if kind is None:
+            raise NotImplementedError("predictive: Categorical and Bernoulli likelihoods only, got %s"
+                                      % type(self.likelihood).__name__)
+        n_samples = int(n_samples)
+        chunk = n_samples if chunk_samples is None else int(chunk_samples)
+        if n_samples < 1 or chunk < 1:
+            raise ValueError("predictive: n_samples and chunk_samples must be positive")
+        batched = self._can_batch() and feat.device.type == "cuda"
+        base, n_local = 0, n_samples
+        if group is not None:
+            if not batched:
+                raise NotImplementedError("predictive: sharding the samples over ranks needs the sample-batched path "
+                                          "(sample_base); this model runs its samples as sequential passes")
+            world = dist.get_world_size(group)
+            if n_samples < world:
+                raise ValueError("predictive: %d samples cannot be sharded over %d ranks" % (n_samples, world))
+            base, n_local = parallel.shard_samples(n_samples, dist.get_rank(group), world)
+        with torch.no_grad():
+            return mc_predictive(self._predictive_chunks(graph, feat, base, n_local, chunk, batched), n_samples, kind,
+                                 y=y, group=group)
+
+    def _predictive_chunks(self, graph, feat, base, n, chunk, batched):
+        if not batched:
+            for _ in range(n):
+                yield self._forward(graph, feat).unsqueeze(0)
+            return
+        # a batched pass reserves the same Philox offsets whatever its sample count, and sample s draws with index
+        # sample_base + s: every chunk starts from the entry state, and after the last one the state is where one
+        # forward(n_samples=n) leaves it
+        seed, offset = _random.get_state()
+        for s0 in range(0, n, chunk):
+            _random._rewind(seed, offset)
+            yield self._forward_samples(graph, feat, min(chunk, n - s0), sample_base=base + s0)
 
     def loss_terms(self, graph, feat, y, mask=None, n_samples=1, kl_scaling=None, sample_base=0):
         """(mean NLL, kl_scaling * mean KL) over ``n_samples`` passes (stag/models.py:63-84)."""

@@ -1087,6 +1087,54 @@ def fused_nll(probs, y, mask=None, kind="categorical"):
     return out[0] if squeeze else out
 
 
+_MC_KIND = {"categorical": 0, "bernoulli": 1}
+
+
+def mc_accumulate(probs, acc_sum, acc_ent, kind="categorical"):
+    """Add the samples of ``probs [S,N,C]`` (float32, unit stride over C; any row / sample strides) to the float64
+    accumulators ``acc_sum [N,C]`` (contiguous) and ``acc_ent [N]`` in sample order (stag_mc_accumulate): the sum of
+    the outputs and the sum of their Categorical / Bernoulli entropies.  No autograd."""
+    _require_cuda(probs, "Monte-Carlo output")
+    lib = _lib.load()
+    dev = probs.device
+    S, N, C = probs.shape
+    if acc_sum.shape != (N, C) or acc_ent.shape != (N,) or acc_sum.dtype != torch.float64 \
+            or acc_ent.dtype != torch.float64 or not acc_sum.is_contiguous() or not acc_ent.is_contiguous():
+        raise ValueError("mc_accumulate: accumulators must be contiguous float64 [N,C] and [N]")
+    pr = probs.detach().to(torch.float32)
+    if pr.stride(-1) != 1 or (N > 1 and pr.stride(1) < C):
+        pr = pr.contiguous()
+    with torch.cuda.device(dev):
+        _lib.check(lib.stag_mc_accumulate(pr.data_ptr(), pr.stride(1) if N > 1 else C, pr.stride(0) if S > 1 else 0,
+                                          N, C, S, _MC_KIND[kind], acc_sum.data_ptr(), acc_ent.data_ptr(),
+                                          _stream(dev)))
+    return acc_sum, acc_ent
+
+
+def mc_finalize(acc_sum, acc_ent, n_samples, kind="categorical", y=None):
+    """(mean [N,C], predictive entropy [N], expected entropy [N], mutual information [N], log-likelihood [N] or None)
+    of ``n_samples`` samples accumulated by :func:`mc_accumulate` (stag_mc_finalize), float32.  ``y``: int64 [N]
+    class labels (Categorical) or [N,C] label values (Bernoulli).  No autograd."""
+    _require_cuda(acc_sum, "Monte-Carlo accumulator")
+    lib = _lib.load()
+    dev = acc_sum.device
+    N, C = acc_sum.shape
+    k = _MC_KIND[kind]
+    yy = None
+    if y is not None:
+        yy = y.to(device=dev, dtype=torch.int64 if k == 0 else torch.float32).contiguous()
+        if tuple(yy.shape) != ((N,) if k == 0 else (N, C)):
+            raise ValueError("mc_finalize: labels of shape %s for outputs [%d, %d]" % (tuple(yy.shape), N, C))
+    mean = torch.empty((N, C), dtype=torch.float32, device=dev)
+    stats = torch.empty((4, N), dtype=torch.float32, device=dev)
+    with torch.cuda.device(dev):
+        _lib.check(lib.stag_mc_finalize(acc_sum.data_ptr(), acc_ent.data_ptr(), N, C, int(n_samples), k, _ptr(yy),
+                                        C if k == 1 else 0, mean.data_ptr(), stats[0].data_ptr(),
+                                        stats[1].data_ptr(), stats[2].data_ptr(),
+                                        stats[3].data_ptr() if yy is not None else 0, _stream(dev)))
+    return mean, stats[0], stats[1], stats[2], (stats[3] if yy is not None else None)
+
+
 class _DenseTransform(torch.autograd.Function):
     """out = act(row_scale * (a @ weight) + bias) on stag_gemm_tcgen05 (3xTF32, fp32 accuracy).
     Backward: dA = g @ W^T through the same kernel, dW / dbias by torch reductions."""

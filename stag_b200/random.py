@@ -72,6 +72,14 @@ def set_state(seed, offset):
         _state["torch_seed"] = int(torch.initial_seed()) & _MASK
 
 
+def _rewind(seed, offset):
+    """Return the stream to a (seed, offset) that ``get_state()`` gave, without moving the device-counter mark as
+    ``set_state`` does: code that replays its own draws (the chunks of ``StagModel.predictive``) stays transparent to
+    ``advance_device_counter``."""
+    with _lock:
+        _state["seed"], _state["offset"] = int(seed) & _MASK, int(offset)
+
+
 def enable_device_counter(device):
     """Create (or return) the device-side call counter of `device`; from now on every launch on that device adds it
     to its Philox counter.  Starts at 0."""
