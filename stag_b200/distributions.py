@@ -130,11 +130,13 @@ class ParametrizedDistribution(Distribution):
     def __init__(self, base_distribution: torch.distributions.Distribution, vi: bool = False):
         super().__init__()
         cls = base_distribution.__class__
-        names = [k for k in base_distribution.arg_constraints.keys() if k != "logits"]
+        # read from the instance: some families (Uniform) define arg_constraints as a property
+        arg_constraints = base_distribution.arg_constraints
+        names = [k for k in arg_constraints.keys() if k != "logits"]
         stored = []
         for name in names:
             value = _as_tensor(getattr(base_distribution, name))
-            if vi and cls.arg_constraints[name] == constraints.positive:
+            if vi and arg_constraints[name] == constraints.positive:
                 setattr(self, "log_" + name, torch.nn.Parameter(torch.log(value)))
                 stored.append("log_" + name)
             elif vi:

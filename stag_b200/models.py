@@ -75,6 +75,66 @@ def mc_predictive(chunks, n_samples, kind, y=None, group=None, accumulate=None, 
     return Predictive(*finalize(acc_sum, acc_ent, n_samples, kind, y), n_samples=int(n_samples))
 
 
+class LossTerms(NamedTuple):
+    """Detached values of the two terms of ``loss_terms``: the mean NLL over the samples and ``kl_scaling`` times the
+    KL."""
+    nll: torch.Tensor
+    reg: torch.Tensor
+
+
+def mc_loss_backward(chunks, n_samples, kl_scaling, group=None, backward=None):
+    """Add to the parameters' ``.grad`` the gradient of the Monte-Carlo objective over ``n_samples`` samples, of which
+    ``chunks`` yields this rank's, in sample order, as ``(c, nll_c, reg_c)``: the chunk's sample count, the sum of its
+    per-sample NLLs and the sum of the vi layers' KL taken right after its forward.  Each chunk's objective
+        ``nll_c / n_samples + (c / n_samples) * kl_scaling * reg_c``
+    is backpropagated and dropped before the next chunk is computed, so memory is that of one chunk.  The KL weights sum
+    to one over the chunks of all ranks: a sample-independent (analytic) KL counts once, and a sample-based one (the
+    fallback of :func:`ops.fused_kl_fallback`, a mean over the chunk's samples) becomes the mean over all samples.
+    With one chunk the expression is the one ``loss_terms`` builds, so the gradients are those of ``loss().backward()``
+    bit for bit.  Returns the :class:`LossTerms` of all samples; with ``group`` the ranks' values are summed by one
+    all-reduce.  ``backward`` (default ``torch.autograd.backward``) is called once per chunk with its objective."""
+    backward = backward or torch.autograd.backward
+    nll_total = reg_total = None
+    for item in chunks:
+        c, nll_c, reg_c = item
+        del item
+        nll = nll_c / n_samples
+        reg = reg_c * (kl_scaling * (c / n_samples))
+        backward(nll + reg)
+        nll = nll.detach()
+        reg = (reg.detach() if torch.is_tensor(reg) else torch.tensor(float(reg))).to(nll)
+        nll_total = nll if nll_total is None else nll_total + nll
+        reg_total = reg if reg_total is None else reg_total + reg
+        del nll_c, reg_c, nll, reg   # before the next chunk is computed: the chunk's graph goes with them
+    if nll_total is None:
+        raise ValueError("Monte-Carlo loss: no samples")
+    values = torch.stack([nll_total, reg_total])
+    if group is not None and dist.get_world_size(group) > 1:
+        dist.all_reduce(values, op=dist.ReduceOp.SUM, group=group)
+    return LossTerms(values[0], values[1])
+
+
+def _shard(what, n_samples, group, batched):
+    """(sample_base, n_local) of this rank's share of ``n_samples``; all of them without ``group``."""
+    if group is None:
+        return 0, n_samples
+    if not batched:
+        raise NotImplementedError("%s: sharding the samples over ranks needs the sample-batched path (sample_base); this "
+                                  "model runs its samples as sequential passes" % what)
+    world = dist.get_world_size(group)
+    if n_samples < world:
+        raise ValueError("%s: %d samples cannot be sharded over %d ranks" % (what, n_samples, world))
+    return parallel.shard_samples(n_samples, dist.get_rank(group), world)
+
+
+def _sample_counts(what, n_samples, chunk_samples):
+    n_samples = int(n_samples)
+    chunk = n_samples if chunk_samples is None else int(chunk_samples)
+    if n_samples < 1 or chunk < 1:
+        raise ValueError("%s: n_samples and chunk_samples must be positive" % what)
+    return n_samples, chunk
+
+
 class StagModel(torch.nn.Module):
     def __init__(self, layers: List[StagLayer], likelihood: Likelihood = CategoricalLikelihood(),
                  kl_scaling=1.0, batch_samples=True):
@@ -161,28 +221,23 @@ class StagModel(torch.nn.Module):
         if kind is None:
             raise NotImplementedError("predictive: Categorical and Bernoulli likelihoods only, got %s"
                                       % type(self.likelihood).__name__)
-        n_samples = int(n_samples)
-        chunk = n_samples if chunk_samples is None else int(chunk_samples)
-        if n_samples < 1 or chunk < 1:
-            raise ValueError("predictive: n_samples and chunk_samples must be positive")
+        n_samples, chunk = _sample_counts("predictive", n_samples, chunk_samples)
         batched = self._can_batch() and feat.device.type == "cuda"
-        base, n_local = 0, n_samples
-        if group is not None:
-            if not batched:
-                raise NotImplementedError("predictive: sharding the samples over ranks needs the sample-batched path "
-                                          "(sample_base); this model runs its samples as sequential passes")
-            world = dist.get_world_size(group)
-            if n_samples < world:
-                raise ValueError("predictive: %d samples cannot be sharded over %d ranks" % (n_samples, world))
-            base, n_local = parallel.shard_samples(n_samples, dist.get_rank(group), world)
+        base, n_local = _shard("predictive", n_samples, group, batched)
+        # sequential passes accumulate one at a time
+        chunks = self._sample_chunks(base, n_local, chunk if batched else 1, batched,
+                                     lambda c, b: self._forward_samples(graph, feat, c, sample_base=b))
         with torch.no_grad():
-            return mc_predictive(self._predictive_chunks(graph, feat, base, n_local, chunk, batched), n_samples, kind,
-                                 y=y, group=group)
+            return mc_predictive(chunks, n_samples, kind, y=y, group=group)
 
-    def _predictive_chunks(self, graph, feat, base, n, chunk, batched):
+    def _sample_chunks(self, base, n, chunk, batched, run):
+        """``run(c, sample_base)`` for consecutive chunks of at most ``chunk`` of this call's ``n`` samples, in sample
+        order, from the Philox state at entry."""
         if not batched:
-            for _ in range(n):
-                yield self._forward(graph, feat).unsqueeze(0)
+            # sequential passes reserve fresh offsets per pass and always draw sample index 0: the chunks continue the
+            # stream as the passes of one call would
+            for s0 in range(0, n, chunk):
+                yield run(min(chunk, n - s0), 0)
             return
         # a batched pass reserves the same Philox offsets whatever its sample count, and sample s draws with index
         # sample_base + s: every chunk starts from the entry state, and after the last one the state is where one
@@ -190,12 +245,10 @@ class StagModel(torch.nn.Module):
         seed, offset = _random.get_state()
         for s0 in range(0, n, chunk):
             _random._rewind(seed, offset)
-            yield self._forward_samples(graph, feat, min(chunk, n - s0), sample_base=base + s0)
+            yield run(min(chunk, n - s0), base + s0)
 
-    def loss_terms(self, graph, feat, y, mask=None, n_samples=1, kl_scaling=None, sample_base=0):
-        """(mean NLL, kl_scaling * mean KL) over ``n_samples`` passes (stag/models.py:63-84)."""
-        if kl_scaling is None:
-            kl_scaling = self.kl_scaling
+    def _sample_terms(self, graph, feat, y, mask, n_samples, sample_base):
+        """(sum of the per-sample NLLs, sum of the vi layers' KL after the forward) of ``n_samples`` passes."""
         outs = self._forward_samples(graph, feat, n_samples, sample_base=sample_base)
         if hasattr(self.likelihood, "nll_samples"):
             # all samples in one fused pass on CUDA (stag_nll), torch.distributions otherwise
@@ -211,11 +264,53 @@ class StagModel(torch.nn.Module):
         for layer in self.layers:
             if layer.vi:
                 reg = reg + layer.kl_divergence()
+        return total_nll, reg
+
+    def loss_terms(self, graph, feat, y, mask=None, n_samples=1, kl_scaling=None, sample_base=0):
+        """(mean NLL, kl_scaling * mean KL) over ``n_samples`` passes (stag/models.py:63-84)."""
+        if kl_scaling is None:
+            kl_scaling = self.kl_scaling
+        total_nll, reg = self._sample_terms(graph, feat, y, mask, n_samples, sample_base)
         # the reference re-evaluates the (sample-independent, analytic) KL once per pass and
         # averages: the mean of n identical terms
         total_nll = total_nll / n_samples
         total_reg = reg * kl_scaling
         return total_nll, total_reg
+
+    def _loss_chunks(self, graph, feat, y, mask, base, n, chunk, batched):
+        return self._sample_chunks(base, n, chunk, batched,
+                                   lambda c, b: (c,) + self._sample_terms(graph, feat, y, mask, c, b))
+
+    def loss_backward(self, graph, feat, y, mask=None, n_samples=1, chunk_samples=None, kl_scaling=None, group=None):
+        """Add to every parameter's ``.grad`` the gradient that ``loss(graph, feat, y, mask, n_samples,
+        kl_scaling).backward()`` adds, running the samples ``chunk_samples`` at a time (all at once when None): each
+        chunk is backpropagated and freed before the next one runs, so peak memory is that of one chunk whatever
+        ``n_samples``.  Returns the detached :class:`LossTerms` ``(nll, reg)`` that ``loss_terms`` returns.
+
+        * The samples are those of ``loss(n_samples=n_samples)`` from the same Philox state, and the state is left
+          where that call and its backward leave it (as in :meth:`predictive`).  Chunks agree with the whole batch to
+          rounding, not bit for bit (the dense transform picks its split-K from the row count); with one chunk the
+          gradients are bitwise those of ``loss().backward()``.
+        * Chunk objective: ``nll_c / n_samples + (c / n_samples) * kl_scaling * reg_c`` (:func:`mc_loss_backward`).
+        * Feature-only layers see each layer's samples in sample order, so BatchNorm running statistics end where
+          ``loss()`` leaves them.  Dropout masks come from torch's RNG, whose draws are ordered by chunk: with dropout
+          the gradients agree with those of ``loss()`` in distribution only.
+        * Models that run their samples as sequential passes (GatedGCN, amortised posteriors, vi with norm,
+          ``batch_samples=False``) run ``chunk_samples`` passes per chunk; ``chunk_samples=1`` holds one pass.  Where
+          the KL depends on the pass (an amortised posterior conditioned on stochastic features), each chunk weights
+          the KL of its last pass: with ``chunk_samples=1`` that is the per-pass mean the reference's loop takes,
+          with one chunk it is the KL of the last pass, as ``loss_terms`` takes it.
+        * ``group``: rank r runs ``parallel.shard_samples(n_samples, r, world)`` (common seed) and scales its terms by
+          the global ``n_samples``, so the SUM of the ranks' gradients is the full gradient: finish the step with one
+          ``parallel.GradBucket.allreduce(average=False)``.  The returned values are summed over the ranks by one
+          all-reduce.  Sequential-pass models cannot shard and raise ``NotImplementedError``."""
+        n_samples, chunk = _sample_counts("loss_backward", n_samples, chunk_samples)
+        if kl_scaling is None:
+            kl_scaling = self.kl_scaling
+        batched = self._can_batch() and feat.device.type == "cuda"
+        base, n_local = _shard("loss_backward", n_samples, group, batched)
+        return mc_loss_backward(self._loss_chunks(graph, feat, y, mask, base, n_local, chunk, batched), n_samples,
+                                kl_scaling, group=group)
 
     def loss(self, graph, feat, y, mask=None, n_samples=1, kl_scaling=None, sample_base=0):
         nll, reg = self.loss_terms(graph, feat, y, mask=mask, n_samples=n_samples, kl_scaling=kl_scaling,
@@ -254,6 +349,10 @@ class StagModelContrastive(StagModel):
             total_nll = total_nll + nll.mean()
             total_reg = total_reg + reg
         return total_nll / n_samples, total_reg / n_samples * kl_scaling
+
+    def loss_backward(self, *args, **kwargs):
+        raise NotImplementedError("StagModelContrastive.loss_backward: the passes return (output, contrastive term) "
+                                  "tuples; use loss().backward()")
 
     def forward(self, graph, feat, n_samples=1, return_parameters=False):
         feat = torch.stack([self._forward(graph, feat)[0] for _ in range(n_samples)], dim=0).mean(dim=0)
