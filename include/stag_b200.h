@@ -350,6 +350,39 @@ STAG_API int stag_mc_finalize(const double* acc_sum, const double* acc_ent, int6
                      int kind, const void* y, int64_t ldy, float* mean, float* pred_entropy, float* exp_entropy,
                      float* mutual_info, float* loglik, void* stream);
 
+/* Calibration of [N,C] probabilities (e.g. the Monte-Carlo mean of stag_mc_finalize) as an int64 table of counts and
+ * fixed-point sums, fx(x) = x * STAG_CAL_ONE rounded half-to-even.  Integer sums do not depend on their order: the
+ * table of a call is the same every run, and the sum of the tables of several calls (row chunks, minibatches, ranks)
+ * is the table of one call over all their rows, bit for bit.  ECE, Brier score, accuracy / micro-F1 and reliability
+ * diagrams follow from the table (stag_b200/calibration.py).
+ *   probs float32 [N,C], row stride ld >= C; mask uint8 [N] or NULL (rows with mask == 0 are not read);
+ *   kind 0 (Categorical): y int64 [N]; kind 1 (Bernoulli): y float32 [N,C], row stride ldy >= C (as stag_mc_finalize);
+ *   table int64 [stag_calibration_table_len(C, n_bins)], caller-owned and caller-zeroed: the call ADDS to it.
+ * Bins (B = n_bins in [1, 64]) are those of sklearn's calibration_curve(strategy="uniform"): interior edges
+ * i * (1.0 / B) (double, i = 1 .. B-1, the values of np.linspace(0, 1, B+1)); bin(x) = the number of interior edges
+ * strictly below x, so bins are (lo, hi] and 0 falls in bin 0.
+ * Layout (int64):
+ *   [0] n: valid rows          [1] n_invalid: rows refused (see below)
+ *   [2] Categorical: rows whose argmax is the label; Bernoulli: tp      [3] 0 | fp      [4] 0 | fn
+ *   [5] brier: sum of fx((q_c - [c == y])^2) over the classes of valid rows (Categorical), of fx((p - y)^2) over the
+ *       labels (Bernoulli)
+ *   [6 ..)         top-label table [3][B]: count, sum of fx(conf), count of correct rows   (Categorical; 0 for Bernoulli)
+ *   [6 + 3B ..)    per-class table [3][C][B]: count, sum of fx(q_c) | fx(p_c), label sum: [c == y] (a count,
+ *                  Categorical) | fx(y_c) (Bernoulli)
+ * Categorical row m (read as doubles): invalid if any m_c is NaN, infinite or negative, if s = sum m_c is 0 or if
+ *   y is outside [0, C).  s is summed as stag_mc_finalize sums a row (lane l of a warp adds classes l, l+32, ... in
+ *   order, then an xor butterfly over offsets 16, 8, 4, 2, 1).  q_c = m_c / s; k = the first index of the largest m_c
+ *   (torch.argmax); conf = q_k; bin(conf) in the top-label table, bin(q_c) in the table of class c.
+ * Bernoulli row: invalid if any p_c or y_c is NaN or outside [0, 1]; tp / fp / fn compare p > 0.5 with y > 0.5;
+ *   bin(p_c) in the table of class c.
+ * Every fixed-point term is at most STAG_CAL_ONE = 2^32: the caller keeps entries below 2^63 by adding at most 2^31
+ * terms to one; one call takes N*C < 2^31 (STAG_EINVAL above).  C <= 1024 (STAG_EUNSUPPORTED above); N = 0 is a no-op.
+ * stag_calibration_table_len: 6 + 3B + 3CB, or STAG_EINVAL for C < 1 or n_bins outside [1, 64]. */
+#define STAG_CAL_ONE 4294967296.0 /* fixed-point unit of the probability sums: 2^32 */
+STAG_API int64_t stag_calibration_table_len(int32_t C, int32_t n_bins);
+STAG_API int stag_calibration(const float* probs, int64_t ld, int64_t N, int32_t C, int kind, const void* y,
+                              int64_t ldy, const uint8_t* mask, int32_t n_bins, int64_t* table, void* stream);
+
 /* Dense feature transform agg @ W (stag/zoo/gcn.py:97-98) on tcgen05 tensor cores with TMEM
  * accumulators; fp32 in / fp32 out computed as 3xTF32 (fp32-level accuracy), fused epilogue
  *   out[m,n] = act( row_scale[m] * sum_k a[m,k]*w[k,n] + bias[n] ),  act: 0 none, 1 relu.

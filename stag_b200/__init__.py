@@ -7,7 +7,7 @@ CUDA behind the C ABI of ``include/stag_b200.h``).  There is no CPU fallback: op
 raise ``StagLibraryError`` when the library is missing or a tensor is not on a CUDA device.
 """
 from . import _lib, random  # noqa: F401
-from . import distributions, likelihoods, utils, graph, function, ops  # noqa: F401
+from . import distributions, likelihoods, utils, graph, function, ops, calibration  # noqa: F401
 from . import layers, models, zoo  # noqa: F401
 from .graph import (Graph, as_graph, batch, rand_graph, add_self_loop, remove_self_loop,  # noqa: F401
                     add_reverse_edges, sum_nodes, mean_nodes)

@@ -98,6 +98,8 @@ SIGNATURES = {
     "stag_nll": (_I, [_V, _I64, _I64, _I64, _I32, _I32, _I, _V, _I64, _V, _V, _V, _V, _V, _SZ, _V]),
     "stag_mc_accumulate": (_I, [_V, _I64, _I64, _I64, _I32, _I32, _I, _V, _V, _V]),
     "stag_mc_finalize": (_I, [_V, _V, _I64, _I32, _I64, _I, _V, _I64, _V, _V, _V, _V, _V, _V]),
+    "stag_calibration_table_len": (_I64, [_I32, _I32]),
+    "stag_calibration": (_I, [_V, _I64, _I64, _I32, _I, _V, _I64, _V, _I32, _V, _V]),
     "stag_gemm_workspace_bytes": (_SZ, [_I64, _I32, _I32]),
     "stag_gemm_tcgen05": (_I, [_V, _I64, _V, _I64, _I64, _I32, _I32, _V, _V, _I, _V, _I64, _V, _SZ, _V]),
     "stag_aggregate_host": (_I, [_I, _V, _V, _I64, _I64, _V, _V, _I32, _I32, _NP, _I, _V, _V]),

@@ -14,7 +14,7 @@ from typing import List, NamedTuple, Optional
 import torch
 import torch.distributed as dist
 
-from . import ops, parallel, random as _random
+from . import calibration as _calibration, ops, parallel, random as _random
 from .layers import StagLayer
 from .likelihoods import Likelihood, CategoricalLikelihood
 from .graph import as_graph
@@ -229,6 +229,18 @@ class StagModel(torch.nn.Module):
                                      lambda c, b: self._forward_samples(graph, feat, c, sample_base=b))
         with torch.no_grad():
             return mc_predictive(chunks, n_samples, kind, y=y, group=group)
+
+    def calibration(self, probs, y, mask=None, n_bins=15):
+        """:class:`stag_b200.calibration.Calibration` of the predictions ``probs [N,C]`` against the labels ``y``
+        (``y [N]`` class indices for a Categorical likelihood, ``[N,C]`` label values for a Bernoulli one) over the rows
+        where ``mask`` is set, in ``n_bins`` equal-width bins: ECE, reliability diagram, Brier score and accuracy /
+        micro-F1, e.g. ``model.calibration(model.predictive(g, x, 256, 32).mean, y, mask=test_mask)``.  The table adds
+        over minibatches (``+``) and ranks (``all_reduce``) exactly."""
+        kind = getattr(self.likelihood, "fused_kind", None)
+        if kind is None:
+            raise NotImplementedError("calibration: Categorical and Bernoulli likelihoods only, got %s"
+                                      % type(self.likelihood).__name__)
+        return _calibration.calibration(probs, y, kind, n_bins=n_bins, mask=mask)
 
     def _sample_chunks(self, base, n, chunk, batched, run):
         """``run(c, sample_base)`` for consecutive chunks of at most ``chunk`` of this call's ``n`` samples, in sample

@@ -1135,6 +1135,61 @@ def mc_finalize(acc_sum, acc_ent, n_samples, kind="categorical", y=None):
     return mean, stats[0], stats[1], stats[2], (stats[3] if yy is not None else None)
 
 
+def calibration_table_len(n_classes, n_bins):
+    """Length of the int64 calibration table of ``n_classes`` classes and ``n_bins`` bins (stag_calibration_table_len):
+    ``6 + 3 n_bins + 3 n_classes n_bins``."""
+    n = _lib.load().stag_calibration_table_len(int(n_classes), int(n_bins))
+    if n < 0:
+        raise _lib.StagError(int(n), "calibration table: n_classes=%d, n_bins=%d (n_bins in [1, 64])"
+                             % (n_classes, n_bins))
+    return n
+
+
+def calibration_table(probs, y, kind="categorical", n_bins=15, mask=None, out=None):
+    """Add the calibration table of ``probs [N,C]`` (float32, unit stride over C) against labels ``y`` (int [N] for
+    ``kind='categorical'``, [N,C] label values for ``'bernoulli'``) to ``out`` (int64, zeroed when None) and return it
+    (stag_calibration; layout in include/stag_b200.h, metrics in :mod:`stag_b200.calibration`).  ``mask``: bool / uint8
+    [N]; rows where it is 0 are not read.  Tables add: the sum of the tables of row chunks is the table of all rows, bit
+    for bit.  No autograd."""
+    _require_cuda(probs, "calibration probabilities")
+    lib = _lib.load()
+    dev = probs.device
+    k = _MC_KIND[kind]
+    if probs.dim() != 2 or probs.dtype != torch.float32:
+        raise ValueError("calibration_table: probabilities must be float32 [N, C], got %s %s"
+                         % (probs.dtype, tuple(probs.shape)))
+    N, C = probs.shape
+    if k == 0:
+        if y.dtype.is_floating_point or y.dtype == torch.bool or y.is_complex():
+            raise ValueError("calibration_table: categorical labels must be integer class indices, got %s" % y.dtype)
+        yy = y.to(device=dev, dtype=torch.int64).contiguous()
+    else:
+        yy = y.to(device=dev, dtype=torch.float32)
+        if yy.dim() == 2 and (yy.stride(-1) != 1 or (N > 1 and yy.stride(0) < C)):
+            yy = yy.contiguous()
+    if tuple(yy.shape) != ((N,) if k == 0 else (N, C)):
+        raise ValueError("calibration_table: labels of shape %s for probabilities [%d, %d]" % (tuple(y.shape), N, C))
+    mk = None
+    if mask is not None:
+        if tuple(mask.shape) != (N,) or mask.dtype not in (torch.bool, torch.uint8):
+            raise ValueError("calibration_table: mask must be bool or uint8 [%d], got %s %s"
+                             % (N, mask.dtype, tuple(mask.shape)))
+        mk = mask.to(device=dev, dtype=torch.uint8).contiguous()
+    n = calibration_table_len(C, n_bins)
+    if out is None:
+        out = torch.zeros(n, dtype=torch.int64, device=dev)
+    elif out.shape != (n,) or out.dtype != torch.int64 or out.device != dev or not out.is_contiguous():
+        raise ValueError("calibration_table: out must be a contiguous int64 [%d] tensor on %s" % (n, dev))
+    pr = probs.detach()
+    if pr.stride(-1) != 1 or (N > 1 and pr.stride(0) < C):
+        pr = pr.contiguous()
+    with torch.cuda.device(dev):
+        _lib.check(lib.stag_calibration(pr.data_ptr(), pr.stride(0) if N > 1 else C, N, C, k, yy.data_ptr(),
+                                        (yy.stride(0) if N > 1 else C) if k == 1 else 0, _ptr(mk), int(n_bins),
+                                        out.data_ptr(), _stream(dev)))
+    return out
+
+
 class _DenseTransform(torch.autograd.Function):
     """out = act(row_scale * (a @ weight) + bias) on stag_gemm_tcgen05 (3xTF32, fp32 accuracy).
     Backward: dA = g @ W^T through the same kernel, dW / dbias by torch reductions."""
