@@ -35,6 +35,9 @@ constexpr int GTHREADS = 128;
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
+// relu that leaves NaN as NaN, as torch.relu does (fmaxf(NaN, 0) is 0: a diverged row would come out as zeros)
+__device__ __forceinline__ float relu_keep_nan(float y) { return y < 0.f ? 0.f : y; }
+
 __device__ __forceinline__ float to_tf32(float x) {
   uint32_t y;
   asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(y) : "f"(x));
@@ -293,7 +296,7 @@ __global__ void __launch_bounds__(GTHREADS) gemm_tcgen05_kernel(const GemmParams
     for (int j = 0; j < 32; ++j) {
       float y = __uint_as_float(v[j]) * rs;
       if (p.bias && n0 + j < p.Nout) y += __ldg(p.bias + n0 + j);
-      if (p.act == 1) y = fmaxf(y, 0.f);
+      if (p.act == 1) y = relu_keep_nan(y);
       scratch[lane * 33 + j] = y;
     }
     __syncwarp();
@@ -546,7 +549,7 @@ __global__ void __launch_bounds__(G2_THREADS, 1) gemm_tma_kernel(const __grid_co
         const int64_t grow = tile * GM + 32 * q + 4 * r8 + (lane >> 3);
         if (grow < p.M) {
           float4 o4 = make_float4(y[r8].x + b4.x, y[r8].y + b4.y, y[r8].z + b4.z, y[r8].w + b4.w);
-          if (p.act == 1) { o4.x = fmaxf(o4.x, 0.f); o4.y = fmaxf(o4.y, 0.f); o4.z = fmaxf(o4.z, 0.f); o4.w = fmaxf(o4.w, 0.f); }
+          if (p.act == 1) { o4.x = relu_keep_nan(o4.x); o4.y = relu_keep_nan(o4.y); o4.z = relu_keep_nan(o4.z); o4.w = relu_keep_nan(o4.w); }
           float* o = p.out + grow * p.ldo + n0 + cq;
           if (vec_o && n0 + cq + 3 < p.Nout) {
             *reinterpret_cast<float4*>(o) = o4;

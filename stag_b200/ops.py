@@ -1237,12 +1237,16 @@ class _DenseTransform(torch.autograd.Function):
         ga = gw = None
         if ctx.needs_input_grad[0]:
             ga = torch.empty((g2.shape[0], K), dtype=torch.float32, device=dev)
-            # the "W^T" operand of the transposed product dA = g @ W^T is W [K, Nout] itself
+            # the "W^T" operand of the transposed product dA = g @ W^T is W [K, Nout] itself.  The kernel writes at
+            # most 256 output columns, so a wider K runs on 256-row slices of W, each into its columns of dA.
             w = weight.detach().to(torch.float32)
             w = (w.t() if ctx.transposed else w).contiguous()
             with torch.cuda.device(dev):
-                _lib.check(lib.stag_gemm_tcgen05(g2.data_ptr(), Nout, w.data_ptr(), Nout, g2.shape[0], K, Nout,
-                                                 0, 0, 0, ga.data_ptr(), K, 0, 0, _stream(dev)))
+                for j in range(0, K, 256):
+                    kk = min(256, K - j)
+                    _lib.check(lib.stag_gemm_tcgen05(g2.data_ptr(), Nout, w.data_ptr() + 4 * j * Nout, Nout,
+                                                     g2.shape[0], kk, Nout, 0, 0, 0, ga.data_ptr() + 4 * j, K,
+                                                     0, 0, _stream(dev)))
             ga = ga.reshape(ctx.a_shape)
         if ctx.needs_input_grad[1]:
             gw = (g2.t() @ a2) if ctx.transposed else (a2.t() @ g2)
@@ -1252,8 +1256,26 @@ class _DenseTransform(torch.autograd.Function):
 def dense_transform(a, weight, row_scale=None, bias=None, relu=False, transposed=False):
     """``act(row_scale[:,None] * (a @ W) + bias)`` on the tcgen05 tensor-core kernel (3xTF32, fp32-level
     accuracy).  ``weight`` is W [K, Nout] (GraphConv layout) or, with ``transposed=True``, W^T [Nout, K]
-    (torch.nn.Linear layout).  Nout > 256 uses torch.matmul (cuBLAS)."""
-    nout = weight.shape[0] if transposed else weight.shape[1]
+    (torch.nn.Linear layout).  Nout > 256 uses torch.matmul (cuBLAS).
+
+    ``row_scale`` has M = a.numel() / K entries, or a divisor of M that is repeated (an [N] scale shared by the S
+    samples of [S,N,K] features); it takes no gradient.  ``bias`` is [Nout].  Anything else raises ``ValueError``.
+
+    Non-finite inputs: NaN in row i of ``a`` gives NaN in all of output row i, NaN in column j of W NaN in all of
+    output column j (NaN * 0 = NaN, as in a float64 product).  +-Inf in ``a`` or W gives NaN rows / columns, not
+    +-Inf: the 3xTF32 split of an infinite x has lo = x - hi = Inf - Inf.  With ``relu`` NaN stays NaN, as in
+    ``torch.relu``.  Finite inputs above (2 - 2^-11) * 2^127, where the tf32 rounding of the high part overflows,
+    and subnormal inputs are outside the accuracy contract."""
+    nout, k = (weight.shape[0], weight.shape[1]) if transposed else (weight.shape[1], weight.shape[0])
+    if row_scale is not None:
+        m, n = a.numel() // max(k, 1), row_scale.numel()
+        if not (n == m or (n > 0 and m % n == 0)):
+            raise ValueError("dense_transform: row_scale has %d entries for %d rows (neither M nor a divisor of M)"
+                             % (n, m))
+        if row_scale.requires_grad:
+            raise ValueError("dense_transform: row_scale takes no gradient; pass row_scale.detach()")
+    if bias is not None and tuple(bias.shape) != (nout,):
+        raise ValueError("dense_transform: bias must have shape [%d], got %s" % (nout, tuple(bias.shape)))
     if nout > 256:
         out = torch.matmul(a, weight.t() if transposed else weight)
         if row_scale is not None:
